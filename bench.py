@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the b200-bls hot path (BASELINE.json: pairings/s and signatures verified/s vs host CPU).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one batch of 65,536 independent full ate pairings (Miller loop + exact final exponentiation,
 BASELINE config 2) per GPU on synthetic seeded inputs; weak scaling: every rank owns its own batch, no data-path
@@ -9,11 +9,13 @@ collective on this metric (SURVEY.md 8e).  Rank 0 prints ONE JSON line:
   value        pairings/s with inputs resident in HBM, CUDA events over the library streams
   e2e          the same through the C-ABI host-buffer call (pinned HOST buffers: H2D, kernel, D2H in the timed region)
   roofline     integer-multiply roofline: limb products the program executes / measured IMAD.WIDE peak
-  cpu_baseline the reference's own CPU implementation (unmodified, baseline/_ref) on all host cores, bounded sample;
+  cpu_baseline the reference's own CPU implementation (unmodified, oracle/_ref) on all host cores, bounded sample;
                its outputs double as the parity oracle for the sampled indices
   extra        signatures verified/s, BASELINE configs 3 / 4 / 5 at full size with their parity booleans, the
                isolated synchronous call, and -- under N > 1 -- the sharded reductions over BOTH exchange transports
 `--impl reference` times that CPU path alone with the same metric and config.
+`--dump-outputs DIR` writes what the last timed step computed (see dump_outputs) so that two builds can be compared
+output for output: the inputs depend only on the seeds and the rank.
 """
 import argparse
 import hashlib
@@ -37,15 +39,15 @@ WORKLOAD = "config2: 65,536 independent ate pairings (Miller loop + final expone
 
 
 # ---------------------------------------------------------------------------------------------
-# CPU arm: the reference itself (baseline/_ref, installed by tools/install_reference.py), else the oracle port
+# CPU arm: the reference itself (oracle/_ref, installed by tools/install_reference.py), else the oracle port
 # ---------------------------------------------------------------------------------------------
 def cpu_impl_kind():
-    return "reference" if os.path.isdir(os.path.join(ROOT, "baseline", "_ref", "bls_py")) else "port"
+    return "reference" if os.path.isdir(os.path.join(ROOT, "oracle", "_ref", "bls_py")) else "port"
 
 
 def extmod_note():
     try:
-        with open(os.path.join(ROOT, "baseline", "_ref", "STATUS.json")) as fh:
+        with open(os.path.join(ROOT, "oracle", "_ref", "STATUS.json")) as fh:
             return json.load(fh)["extmod"]
     except (OSError, ValueError, KeyError):
         return "extmod: does not build in this image (no gmp.h; CPython-3.12-incompatible int access, SURVEY.md 8c)"
@@ -62,7 +64,7 @@ def _cpu_load(kind):
         import logging
         logging.disable(logging.CRITICAL)          # the reference logs that its Cython accelerator is absent
         sys.dont_write_bytecode = True
-        sys.path.insert(0, os.path.join(ROOT, "baseline", "_ref"))
+        sys.path.insert(0, os.path.join(ROOT, "oracle", "_ref"))
         from bls_py import ec, pairing
         from bls_py.fields import Fq, Fq2
         q = ec.default_ec.q
@@ -163,6 +165,24 @@ def sample_indices(seed, n, k):
     import numpy as np
     rng = np.random.Generator(np.random.PCG64(seed))
     return sorted(int(i) for i in rng.choice(n, size=min(k, n), replace=False))
+
+
+DUMP_ROWS = 16384                # a quarter of the batch: 16,384 x 144 float64 words = 18.9 MB
+
+
+def dump_outputs(path, out):
+    """--dump-outputs: the GT elements of one batch (out: uint8, 576 bytes per pairing = 12 Fq coefficients of 48
+    big-endian bytes) at DUMP_ROWS seeded row indices, written as
+      DIR/pairings.npy         float64 (rows, 12, 12): each coefficient's big-endian 32-bit words, most significant
+                               first (exact: every word < 2^53)
+      DIR/pairing_rows.npy     float64 (rows,): the batch indices of those rows, ascending"""
+    import numpy as np
+    n = out.size // 576
+    rows = np.array(sample_indices(0xD0D0, n, DUMP_ROWS), dtype=np.int64)
+    words = out.view(">u4").reshape(n, 12, 12)[rows]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "pairings.npy"), words.astype(np.float64))
+    np.save(os.path.join(path, "pairing_rows.npy"), rows.astype(np.float64))
 
 
 def run_reference(args, rank):
@@ -318,6 +338,7 @@ def run_gpu(args, rank, world):
     barrier()
     clocks = sampler.stop()
     check(lib.b200bls_set_stream(0))
+    last_out = sets[(args.warmup + args.steps - 1) % NSETS][2].download() if rank == 0 else None
 
     # --- end to end through the host-buffer C ABI call, pinned host memory, one buffer set per stream
     def pinned(nbytes):
@@ -366,10 +387,9 @@ def run_gpu(args, rank, world):
         idx = sample_indices(0xB2C, n, 4 * cores)
         items = [(i, 0, 0, hP[96 * i:96 * (i + 1)].tobytes(), hQ[192 * i:192 * (i + 1)].tobytes()) for i in idx]
         cpu_v, cpu_cores, outs = cpu_pairings(items, cores)
-        dev_out = sets[(args.warmup + args.steps - 1) % NSETS][2].download()
         match = all(aO[576 * i:576 * (i + 1)].tobytes() == outs[i] for i in idx)
         parity = {"sampled_outputs_equal_cpu_%s" % cpu_impl_kind(): bool(match), "samples": len(idx),
-                  "device_path_equals_host_path": bool(np.array_equal(dev_out, aO)),
+                  "device_path_equals_host_path": bool(np.array_equal(last_out, aO)),
                   "isolated_call_equals_streamed": lone_same,
                   "output_sha256": hashlib.sha256(aO.tobytes()).hexdigest()}
         cpu = {"value": cpu_v, "unit": METRIC, "cores": cpu_cores, "kind": cpu_impl_kind(),
@@ -414,6 +434,8 @@ def run_gpu(args, rank, world):
         D.shutdown()
     if rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_out)
     if world > 1:
         time.sleep(1.0)      # let the other ranks' exit chatter (NCCL_DEBUG lines share this stdout) precede the JSON line
     value = world * n * args.steps / (ms * 1e-3)
@@ -608,7 +630,13 @@ def main():
     ap.add_argument("--steps", type=int, default=12)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write rank 0's output of the last timed step as .npy files into DIR (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; --impl reference has none")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":

@@ -59,10 +59,8 @@ def test_no_cpu_fallback():
 
 def test_plugin_seam_signatures_match_the_reference():
     """bls_b200.fields_t_c offers functions of the reference's accelerator seam (fields_t.py:1218-1265)
-    under the same names and parameter lists; checked against the live reference where it is mounted
-    (development container), against the recorded parameter lists elsewhere"""
+    under the same names and parameter lists, recorded from the reference"""
     import inspect
-    import sys
     from bls_b200 import fields_t_c as C
     recorded = {
         "fq_ate_pairing_multi": ["Ps", "Qs"],
@@ -73,15 +71,3 @@ def test_plugin_seam_signatures_match_the_reference():
     }
     for name, params in recorded.items():
         assert list(inspect.signature(getattr(C, name)).parameters) == params, name
-    if os.path.isdir("/root/reference/bls_py"):
-        sys.path.insert(0, "/root/reference")
-        sys.dont_write_bytecode = True
-        import logging
-        logging.disable(logging.CRITICAL)
-        try:
-            from bls_py import fields_t as ref
-        finally:
-            logging.disable(logging.NOTSET)
-            sys.path.remove("/root/reference")
-        for name, params in recorded.items():
-            assert list(inspect.signature(getattr(ref, name)).parameters) == params, name

@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
-"""Reference arm of the benchmark: copies the UNMODIFIED reference package (pure Python) from /root/reference
-into the git-ignored baseline/_ref/ -- it travels to the GPU box with the snapshot like the built .so files, where
-`bench.py --impl reference` and bench.py's cpu_baseline leg import it (kind: "reference").  Nothing is patched and
+"""Reference arm of the benchmark: copies the UNMODIFIED reference package (pure Python) from SRC into the
+git-ignored oracle/_ref/, where `bench.py --impl reference` and bench.py's cpu_baseline leg import it (kind:
+"reference"); without SRC, an oracle/_ref/ already in the tree is kept.  build() runs this.  Nothing is patched and
 no reference source enters the repository's history.  Also records whether the reference's optional Cython + GMP
 accelerator (extmod/) can be built in this image (BASELINE.md section 3).
 
@@ -16,7 +16,7 @@ import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SRC = "/root/reference"
-DST = os.path.join(ROOT, "baseline", "_ref")
+DST = os.path.join(ROOT, "oracle", "_ref")
 
 
 def extmod_status():
@@ -38,7 +38,7 @@ def extmod_status():
 
 def main():
     if not os.path.isdir(os.path.join(SRC, "bls_py")):
-        print("no reference at %s: keeping whatever baseline/_ref holds" % SRC)
+        print("no reference at %s: keeping whatever %s holds" % (SRC, DST))
         return 0
     shutil.rmtree(DST, ignore_errors=True)
     os.makedirs(DST)
