@@ -190,6 +190,19 @@ int b200bls_g2_decompress_batch(const uint8_t* in, uint8_t* out, uint8_t* ok, si
 /* AffinePoint.serialize (ec.py:94-111): affine -> compressed (x, top bit = lex_gt_neg). */
 int b200bls_g1_compress_batch(const uint8_t* in, uint8_t* out, size_t n);
 int b200bls_g2_compress_batch(const uint8_t* in, uint8_t* out, size_t n);
+/* Prime-order subgroup membership, which the reference never checks: ok[i] = 1 iff affine point i
+ * (g2 = 0: 96 bytes, G1; g2 = 1: 192 bytes, G2) lies on the curve and in G1 / G2.  Coordinates are
+ * read mod q, as by every entry point taking affine points; infinity is the identity and counts as a
+ * member, and it is every point whose coordinates reduce to (0, 0): zero bytes, but also q || 0, 0 || q
+ * and q || q per coordinate.  Endomorphism tests (Scott 2021): psi(P) == [x]P on G2,
+ * (beta x, y) == [-x^2]P on G1, about 1.1 k / 1.3 k Montgomery products per point. */
+int b200bls_subgroup_check_batch(int g2, const uint8_t* pts, uint8_t* ok, size_t n);
+int b200bls_subgroup_check_batch_dev(int g2, const void* pts, void* ok, size_t n);
+/* The public-key rule of the strict verifications below (KeyValidate of the IETF BLS draft): ok[i] = 1
+ * iff affine G1 point i (96 bytes) is in G1 and is not infinity, both decided on the coordinates
+ * reduced mod q, as the pairing reads them. */
+int b200bls_key_validate_batch(const uint8_t* pts, uint8_t* ok, size_t n);
+int b200bls_key_validate_batch_dev(const void* pts, void* ok, size_t n);
 
 /* The reference's Jacobian-coordinate functions on JACOBIAN inputs, the granularity of its plugin seam
  * (fields_t.py:1218-1265): a = n x (X, Y, Z), three coordinates of 48 (G1) / 96 (G2) bytes, infinity = Z = 0.
@@ -231,6 +244,17 @@ int b200bls_verify_batch_dev(const void* pk, const void* mh, const void* sig, vo
  * signature that does not decode -- the reference raises ValueError -- gives ok[i] = 0. */
 int b200bls_verify_batch_wire(const uint8_t* pk48, const uint8_t* mh, const uint8_t* sig96, uint8_t* ok, size_t n);
 int b200bls_verify_batch_wire_dev(const void* pk48, const void* mh, const void* sig96, void* ok, size_t n);
+/* Strict forms of b200bls_verify_batch / b200bls_verify_batch_wire: the same verdict AND-ed with
+ * "pk_i is in G1 and is not infinity" and "sig_i is in G2" (b200bls_subgroup_check_batch).  The
+ * reference accepts points outside the subgroups: the order-3 key (0, 2) verifies the infinity
+ * signature for every message, pk + (0, 2) verifies pk's signatures, and the infinity key verifies
+ * the infinity signature.  Rejecting the infinity key is the KeyValidate rule of the IETF BLS draft;
+ * it is decided on the reduced coordinates, so a key encoded as q || 0 is infinity and rejected too. */
+int b200bls_verify_batch_strict(const uint8_t* pk, const uint8_t* mh, const uint8_t* sig, uint8_t* ok, size_t n);
+int b200bls_verify_batch_strict_dev(const void* pk, const void* mh, const void* sig, void* ok, size_t n);
+int b200bls_verify_batch_wire_strict(const uint8_t* pk48, const uint8_t* mh, const uint8_t* sig96, uint8_t* ok,
+                                     size_t n);
+int b200bls_verify_batch_wire_strict_dev(const void* pk48, const void* mh, const void* sig96, void* ok, size_t n);
 /* One aggregate signature over n distinct message hashes (bls.py:194-201):
  * *ok = (e(-G1, sig) * prod_i e(pk_i, H(mh_i)) == 1).  n + 1 Miller loops, one final
  * exponentiation.  pks are the per-message public-key sums the host-side grouping produced. */

@@ -78,6 +78,14 @@ def _load():
         "b200bls_g2_decompress_batch": (i32, [vp, vp, vp, sz]),
         "b200bls_g1_compress_batch": (i32, [vp, vp, sz]),
         "b200bls_g2_compress_batch": (i32, [vp, vp, sz]),
+        "b200bls_subgroup_check_batch": (i32, [i32, vp, vp, sz]),
+        "b200bls_subgroup_check_batch_dev": (i32, [i32, vp, vp, sz]),
+        "b200bls_key_validate_batch": (i32, [vp, vp, sz]),
+        "b200bls_key_validate_batch_dev": (i32, [vp, vp, sz]),
+        "b200bls_verify_batch_strict": (i32, [vp, vp, vp, vp, sz]),
+        "b200bls_verify_batch_strict_dev": (i32, [vp, vp, vp, vp, sz]),
+        "b200bls_verify_batch_wire_strict": (i32, [vp, vp, vp, vp, sz]),
+        "b200bls_verify_batch_wire_strict_dev": (i32, [vp, vp, vp, vp, sz]),
         "b200bls_g1_msm": (i32, [vp, vp, vp, sz]),
         "b200bls_g1_msm_dev": (i32, [vp, vp, vp, sz]),
         "b200bls_g2_msm": (i32, [vp, vp, vp, sz]),

@@ -59,9 +59,10 @@ class BLS:
         return final
 
     @staticmethod
-    def verify(signature):
+    def verify(signature, strict=False):
         """bls.py:154-201: group keys by message, raise each to its exponent from the
-        aggregation tree, one multi-pairing against the hashed messages"""
+        aggregation tree, one multi-pairing against the hashed messages.  strict=True: False as well when the
+        signature is outside G2 or a public key is outside G1 or is infinity (the reference accepts these)"""
         info = signature.aggregation_info
         ec.serialize_many([pk.value for pk in info.public_keys])
         groups = {}
@@ -69,6 +70,12 @@ class BLS:
             groups.setdefault(mh, []).append(pk)
         if not groups:
             raise IndexError("signature has no aggregation info entries")
+        if strict:
+            keys = list(set(info.public_keys))
+            if not signature.value.is_in_subgroup():
+                return False
+            if not engine.key_validate(b"".join(pk.value.raw for pk in keys)).all():
+                return False
         flat_pts, flat_exp, spans = [], [], []
         for mh, pks in groups.items():
             uniq = list(set(pks))
@@ -92,19 +99,21 @@ class BLS:
                                        b"".join(mh for mh, _, _ in spans))
 
     @staticmethod
-    def verify_batch(public_keys, message_hashes, signatures):
+    def verify_batch(public_keys, message_hashes, signatures, strict=False):
         """n independent single-message verifications in one GPU pass -> list of bool
-        (the data-parallel form of calling BLS.verify n times)"""
+        (the data-parallel form of calling BLS.verify n times).  strict=True: False as well for a key outside G1,
+        the infinity key or a signature outside G2"""
         res = engine.verify_batch(b"".join(pk.value.raw for pk in public_keys), b"".join(message_hashes),
-                                  b"".join(s.value.raw for s in signatures))
+                                  b"".join(s.value.raw for s in signatures), strict)
         return [bool(r) for r in res]
 
     @staticmethod
-    def verify_batch_bytes(public_key_bytes, message_hashes, signature_bytes):
+    def verify_batch_bytes(public_key_bytes, message_hashes, signature_bytes, strict=False):
         """the same from serialised keys (48 B) and signatures (96 B): PublicKey.from_bytes /
         Signature.from_bytes run on the GPU too; where the reference would raise ValueError while
-        decoding, the result is False"""
-        res = engine.verify_batch_wire(b"".join(public_key_bytes), b"".join(message_hashes), b"".join(signature_bytes))
+        decoding, the result is False.  strict: as in verify_batch"""
+        res = engine.verify_batch_wire(b"".join(public_key_bytes), b"".join(message_hashes), b"".join(signature_bytes),
+                                       strict)
         return [bool(r) for r in res]
 
     @staticmethod

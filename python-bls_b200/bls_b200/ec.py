@@ -91,6 +91,11 @@ class Point:
     def __hash__(self):
         return hash((self.g2, self.raw))
 
+    def is_in_subgroup(self):
+        """on the curve and in the prime-order subgroup G1 / G2 (infinity is); the reference has no such test.
+        Batches: engine.subgroup_check"""
+        return bool(engine.subgroup_check(self.raw, self.g2)[0])
+
     def serialize(self):
         """x with the 'y is the larger root' flag in the top bit (ec.py:94-111)"""
         if self._ser is None:
@@ -215,23 +220,26 @@ def _canonical_encoding(data, raw, g2):
     return masked
 
 
-def point_from_bytes(data, g2):
+def point_from_bytes(data, g2, check_subgroup=False):
     """PublicKey.from_bytes / Signature.from_bytes decoding (keys.py:29-40, signature.py:22-38);
-    raises ValueError where the reference does"""
+    raises ValueError where the reference does, and with check_subgroup=True also for a point outside G1 / G2"""
     out, ok = engine.decompress(data, g2)
     if not ok[0]:
         raise ValueError("No y for point x")
+    if check_subgroup and not engine.subgroup_check(out, g2)[0]:
+        raise ValueError("point is not in the prime-order subgroup")
     p = Point(out.tobytes(), g2)
     p._ser = _canonical_encoding(bytes(data), p.raw, g2)
     return p
 
 
-def points_from_bytes(buffers, g2):
+def points_from_bytes(buffers, g2, check_subgroup=False):
     """many PublicKey.from_bytes / Signature.from_bytes decodings in ONE GPU call (row f2: the
     reference decodes, and later re-serialises, one key at a time).  The serialised form of each
     point is known at once -- the input with its two spare flag bits cleared (the reference masks
     them on input and never sets them on output) -- so sorting / hashing these points later costs
-    no further GPU work.  Raises ValueError if any buffer does not decode, like the reference."""
+    no further GPU work.  Raises ValueError if any buffer does not decode, like the reference, and with
+    check_subgroup=True also if any point is outside G1 / G2 (one more batched call)."""
     buffers = [bytes(b) for b in buffers]
     if not buffers:
         return []
@@ -239,6 +247,10 @@ def points_from_bytes(buffers, g2):
     out, ok = engine.decompress(b"".join(buffers), g2)
     if not ok.all():
         raise ValueError("No y for point x (buffer %d)" % int(np.argmin(ok)))
+    if check_subgroup:
+        member = engine.subgroup_check(out, g2)
+        if not member.all():
+            raise ValueError("point is not in the prime-order subgroup (buffer %d)" % int(np.argmin(member)))
     raw = out.tobytes()
     pts = []
     for i, b in enumerate(buffers):

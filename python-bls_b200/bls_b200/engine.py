@@ -230,6 +230,34 @@ def decompress(data, g2):
     return out, ok
 
 
+def subgroup_check(points, g2):
+    """n affine points (96 / 192 B) -> n flag bytes: 1 iff the point is on the curve and in G1 / G2.  Coordinates are
+    read mod q like every affine input here, and infinity counts as a member: any coordinates that reduce to (0, 0),
+    zero bytes as well as q per coordinate"""
+    _lib.init()
+    w = _g(g2)[1]
+    points = as_u8(points)
+    n = points.size // w
+    if points.size != n * w:
+        raise ValueError("bad buffer size")
+    ok = np.empty(n, dtype=np.uint8)
+    check(lib.b200bls_subgroup_check_batch(int(bool(g2)), ptr(points), ptr(ok), n))
+    return ok
+
+
+def key_validate(points):
+    """n affine G1 points (96 B) -> n flag bytes: 1 iff the point is in G1 and is not infinity (the public-key rule of
+    strict verification), decided on the coordinates reduced mod q"""
+    _lib.init()
+    points = as_u8(points)
+    n = points.size // 96
+    if points.size != n * 96:
+        raise ValueError("bad buffer size")
+    ok = np.empty(n, dtype=np.uint8)
+    check(lib.b200bls_key_validate_batch(ptr(points), ptr(ok), n))
+    return ok
+
+
 def compress(points, g2):
     _lib.init()
     name, w = _g(g2)
@@ -292,28 +320,32 @@ def aggregate_miller(sig, pks, hashes):
     return out
 
 
-def verify_batch_wire(pks48, hashes, sigs96):
+def verify_batch_wire(pks48, hashes, sigs96, strict=False):
     """n x (serialised pk 48 B, message hash 32 B, serialised sig 96 B) -> n result bytes; inputs that
-    do not decode are rejections"""
+    do not decode are rejections.  strict=True: also rejects keys outside G1, the infinity key and
+    signatures outside G2 (the reference accepts them)"""
     _lib.init()
     pks48, hashes, sigs96 = as_u8(pks48), as_u8(hashes), as_u8(sigs96)
     n = hashes.size // 32
     if pks48.size != 48 * n or hashes.size != 32 * n or sigs96.size != 96 * n:
         raise ValueError("bad buffer sizes")
     out = np.empty(n, dtype=np.uint8)
-    check(lib.b200bls_verify_batch_wire(ptr(pks48), ptr(hashes), ptr(sigs96), ptr(out), n))
+    fn = lib.b200bls_verify_batch_wire_strict if strict else lib.b200bls_verify_batch_wire
+    check(fn(ptr(pks48), ptr(hashes), ptr(sigs96), ptr(out), n))
     return out
 
 
-def verify_batch(pks, hashes, sigs):
-    """n x (pk 96 B, message hash 32 B, sig 192 B) -> n result bytes"""
+def verify_batch(pks, hashes, sigs, strict=False):
+    """n x (pk 96 B, message hash 32 B, sig 192 B) -> n result bytes.  strict=True: also rejects keys
+    outside G1, the infinity key and signatures outside G2 (the reference accepts them)"""
     _lib.init()
     pks, hashes, sigs = as_u8(pks), as_u8(hashes), as_u8(sigs)
     n = hashes.size // 32
     if pks.size != 96 * n or hashes.size != 32 * n or sigs.size != 192 * n:
         raise ValueError("bad buffer sizes")
     ok = np.empty(n, dtype=np.uint8)
-    check(lib.b200bls_verify_batch(ptr(pks), ptr(hashes), ptr(sigs), ptr(ok), n))
+    fn = lib.b200bls_verify_batch_strict if strict else lib.b200bls_verify_batch
+    check(fn(ptr(pks), ptr(hashes), ptr(sigs), ptr(ok), n))
     return ok
 
 

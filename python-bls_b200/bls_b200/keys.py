@@ -14,13 +14,14 @@ class PublicKey:
         self.value = value                      # ec.Point on G1
 
     @staticmethod
-    def from_bytes(buffer):
-        return PublicKey(ec.point_from_bytes(bytes(buffer), False))
+    def from_bytes(buffer, check_subgroup=False):
+        """check_subgroup=True: ValueError also for a point outside G1 (the reference accepts it)"""
+        return PublicKey(ec.point_from_bytes(bytes(buffer), False, check_subgroup))
 
     @staticmethod
-    def from_bytes_batch(buffers):
+    def from_bytes_batch(buffers, check_subgroup=False):
         """many keys decoded in one GPU call; their serialised forms are cached"""
-        return [PublicKey(p) for p in ec.points_from_bytes(buffers, False)]
+        return [PublicKey(p) for p in ec.points_from_bytes(buffers, False, check_subgroup)]
 
     @staticmethod
     def from_g1(g1_el):

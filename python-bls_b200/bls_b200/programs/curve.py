@@ -18,6 +18,10 @@ G1_GEN = (int("17f1d3a73197d7942695638c4fa9ac0fc3688c4f9774b905a14e3a3f171bac58"
               "6c55e83ff97a1aeffb3af00adb22c6bb", 16),
           int("08b3f481e3aaa0f1a09e30ed741d8ae4fcf5e095d5d00af600db18cb2c04b3ed"
               "d03cc744a2888ae40caa232946c5e7e1", 16))
+# phi(x, y) = (BETA x, y) acts on G1 as [-x^2] (x the BLS parameter); the other primitive cube root of unity, BETA^2,
+# gives the eigenvalue x^2 - 1 instead
+BETA = 0x5f19672fdf76ce51ba69c6076a0f77eaddb3a93be6f89688de17d813620a00022e01fffffffefffe
+assert pow(BETA, 3, Q) == 1 and BETA != 1
 
 
 class Curve:
@@ -221,6 +225,33 @@ class Curve:
             nz = d1 | d0
             acc = tuple(self.sel(nz, a, b) for a, b in zip(s, acc))
         return acc
+
+    def subgroup_ladder(self, x, y, inf):
+        """the Jacobian multiple in_subgroup compares with the endomorphism image: [|x|] P on G2, [x^2] P =
+        [|x|]([|x|] P) on G1.  Complete additions: on a point of small order the accumulator can equal P at an
+        addition step (the order-3 and order-11 points of E(Fq) do)."""
+        from .hashg2 import mul_by_x_abs
+        acc = mul_by_x_abs(self, (x, y), complete=True, inf=inf)
+        return acc if self.g2 else mul_by_x_abs(self, acc, complete=True)
+
+    def in_subgroup(self, x, y, inf):
+        """flag: the affine point is on the curve and in the prime-order subgroup (infinity is).  Endomorphism tests
+        (Scott, "A note on group membership tests for G1, G2 and GT on BLS pairing-friendly curves", 2021):
+        G2: psi(P) == [x] P = -[|x|] P;  G1: phi(P) == -[x^2] P = -[|x|]([|x|] P).
+        The ladder result (X, Y, Z) is compared with the affine image (x', y') projectively: X == x' Z^2,
+        Y == -y' Z^3, Z != 0.  The curve equation is checked too: the doubling formulas never use b, so an
+        off-curve point would be tested on another curve."""
+        from .hashg2 import PSI_CX, PSI_CY, B2
+        prog = self.prog
+        on_curve = y.sqr().eq(x.sqr() * x + self.const(B2 if self.g2 else 4))
+        X, Y, Z = self.subgroup_ladder(x, y, inf)
+        if self.g2:
+            xi, yi = x.conj() * prog.const2(PSI_CX), y.conj() * prog.const2(PSI_CY)
+        else:
+            xi, yi = x * prog.const1(BETA), y
+        zz = Z.sqr()
+        same = X.eq(xi * zz) & (-Y).eq(yi * (zz * Z)) & ~Z.is_zero()
+        return inf | (on_curve & same)
 
 
 # ---------------------------------------------------------------------------------------
@@ -597,6 +628,23 @@ def build_decompress(g2):
             prog.store1_be48(1, 0, prog.sel1(ok, x, zero))
             prog.store1_be48(1, 48, prog.sel1(ok, y, zero))
         prog.store_flag(2, 0, ok)
+        return prog
+    return build
+
+
+def build_subgroup_check(g2, key=False):
+    """buffers: 0 = affine points (96 / 192 B), 1 = flag byte: 1 iff the point is on the curve and in G1 / G2
+    (Curve.in_subgroup; infinity counts as a member).  Coordinates are read mod q like every affine input, so
+    infinity is any pair of coordinates that reduces to (0, 0): zero bytes, and also q || 0, 0 || q, q || q.
+    key=True (G1, "g1_keyvalidate"): the public-key rule of strict verification, a member that is NOT infinity,
+    decided on the same reduced coordinates.  The reference checks neither."""
+    def build():
+        prog = Program("g1_keyvalidate" if key else ("g2_subgroup" if g2 else "g1_subgroup"))
+        prog.begin_body()
+        c = Curve(prog, g2)
+        x, y, inf = c.load_affine(0)
+        f = c.in_subgroup(x, y, inf)
+        prog.store_flag(1, 0, f & ~inf if key else f)
         return prog
     return build
 

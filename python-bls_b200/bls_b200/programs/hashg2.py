@@ -148,13 +148,16 @@ def psi2(prog, p):
     return (x * prog.const1(PSI2_CX), -y, z)
 
 
-def mul_by_x_abs(c, p):
-    """|x| * P, fixed scalar, MSB first"""
-    acc = p
+def mul_by_x_abs(c, p, complete=False, inf=None):
+    """|x| * P, fixed scalar, MSB first.  With `inf` given, P = (x, y) is affine with that infinity flag and the
+    additions are mixed.  complete=False leaves P + P out of the additions, which is exact while the accumulator
+    cannot equal P (P of large order, as in the cofactor clearing); points of small order need complete=True."""
+    mixed = inf is not None
+    acc = c.from_affine(p[0], p[1], inf) if mixed else p
     for bit in bin(X_ABS)[3:]:
         acc = c.double(acc)
         if bit == "1":
-            acc = c.add(acc, p, complete=False)
+            acc = c.add(acc, p, mixed=mixed, inf2=inf, complete=complete)
     return acc
 
 

@@ -67,6 +67,8 @@ for _g2 in (False, True):
     for _op in ("affine", "dbl", "add", "mul"):        # the plugin seam's Jacobian-coordinate functions
         PROGRAMS[_p + "_j" + _op] = curve.build_jacobian_op(_g2, _op)
     PROGRAMS[_p + "_cflag"] = curve.build_compress_flag(_g2)
+    PROGRAMS[_p + "_subgroup"] = curve.build_subgroup_check(_g2)
+PROGRAMS["g1_keyvalidate"] = curve.build_subgroup_check(False, key=True)
 
 
 # programs assembled for the one-CTA-per-SM shape only (seam / parity utilities, never launched in bulk)

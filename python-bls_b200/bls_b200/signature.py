@@ -11,13 +11,14 @@ class Signature:
         self.aggregation_info = aggregation_info
 
     @staticmethod
-    def from_bytes(buffer, aggregation_info=None):
-        return Signature(ec.point_from_bytes(bytes(buffer), True), aggregation_info)
+    def from_bytes(buffer, aggregation_info=None, check_subgroup=False):
+        """check_subgroup=True: ValueError also for a point outside G2 (the reference accepts it)"""
+        return Signature(ec.point_from_bytes(bytes(buffer), True, check_subgroup), aggregation_info)
 
     @staticmethod
-    def from_bytes_batch(buffers):
+    def from_bytes_batch(buffers, check_subgroup=False):
         """many signatures decoded in one GPU call (no aggregation info attached)"""
-        return [Signature(p) for p in ec.points_from_bytes(buffers, True)]
+        return [Signature(p) for p in ec.points_from_bytes(buffers, True, check_subgroup)]
 
     @staticmethod
     def from_g2(g2_el, aggregation_info=None):

@@ -774,15 +774,71 @@ int verify_dev(const void* pk, const void* mh, const void* sig, void* ok, size_t
   return launch_named("verify_full", n, b, 4);
 }
 
-__global__ void and3_kernel(uint8_t* __restrict__ ok, const uint8_t* __restrict__ a, const uint8_t* __restrict__ b, long long n) {
+// one flag byte per affine point from a g?_subgroup-style program (programs/curve.py: build_subgroup_check)
+int point_flags_dev(const char* program, bool g2, const void* pts, void* ok, size_t n) {
+  NEED_READY();
+  if (n == 0) return 0;
+  VmBuf b[2] = {vb(pts, g2 ? 192 : 96), vb(ok, 1)};
+  return launch_named(program, n, b, 2);
+}
+
+// ok[i] = 1 iff point i is on the curve and in G1 / G2 (Curve.in_subgroup; infinity counts as a member)
+int subgroup_check_dev(bool g2, const void* pts, void* ok, size_t n) {
+  return point_flags_dev(g2 ? "g2_subgroup" : "g1_subgroup", g2, pts, ok, n);
+}
+
+struct FlagList {
+  const uint8_t* f[4];
+  int n;
+};
+
+// ok[i] &= byte i of every flag array
+__global__ void and_flags_kernel(uint8_t* __restrict__ ok, FlagList fl, long long n) {
   long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (t < n) ok[t] = (ok[t] && a[t] && b[t]) ? 1 : 0;
+  if (t >= n) return;
+  bool v = ok[t] != 0;
+#pragma unroll
+  for (int i = 0; i < 4; i++)
+    if (i < fl.n) v = v && fl.f[i][t];
+  ok[t] = v ? 1 : 0;
+}
+
+int and_flags_dev(void* ok, const FlagList& fl, size_t n) {
+  and_flags_kernel<<<(unsigned)((n + 255) / 256), 256, 0, STREAM>>>((uint8_t*)ok, fl, (long long)n);
+  CU(cudaGetLastError());
+  g_ctx.launches++;
+  return 0;
+}
+
+// strict verification: "pk in G1 and not infinity" (g1_keyvalidate, decided on the coordinates reduced mod q as the
+// pairing reads them) and "sig in G2" for the affine keys and signatures into scratch[13], appended to fl
+int strict_flags_dev(const void* pk, const void* sig, size_t n, FlagList& fl) {
+  int rc = ensure_scratch(13, 2 * n);
+  if (rc) return rc;
+  uint8_t* f = (uint8_t*)cur().scratch[13].ptr;
+  rc = point_flags_dev("g1_keyvalidate", false, pk, f, n);
+  if (!rc) rc = subgroup_check_dev(true, sig, f + n, n);
+  fl.f[fl.n++] = f;
+  fl.f[fl.n++] = f + n;
+  return rc;
+}
+
+// strict: the verdict AND-ed with "pk in G1, pk not infinity, sig in G2" (b200bls.h)
+int verify_strict_dev(const void* pk, const void* mh, const void* sig, void* ok, size_t n) {
+  NEED_READY();
+  if (n == 0) return 0;
+  int rc = verify_dev(pk, mh, sig, ok, n);
+  FlagList fl = {};
+  if (!rc) rc = strict_flags_dev(pk, sig, n, fl);
+  if (rc) return rc;
+  return and_flags_dev(ok, fl, n);
 }
 
 // verification straight from the wire formats: PublicKey.from_bytes (keys.py:29-40) and
 // Signature.from_bytes (signature.py:22-38) on the device, then the pairing check; a key or
-// signature that does not decode (the reference raises ValueError) counts as a rejection
-int verify_wire_dev(const void* pk48, const void* mh, const void* sig96, void* ok, size_t n) {
+// signature that does not decode (the reference raises ValueError) counts as a rejection.
+// strict: the subgroup checks of verify_strict_dev on the decoded points as well.
+int verify_wire_dev(const void* pk48, const void* mh, const void* sig96, void* ok, size_t n, bool strict = false) {
   NEED_READY();
   if (n == 0) return 0;
   int rc = ensure_scratch(6, (size_t)96 * n);
@@ -799,11 +855,12 @@ int verify_wire_dev(const void* pk48, const void* mh, const void* sig96, void* o
   if (rc) return rc;
   rc = verify_dev(sc.scratch[6].ptr, mh, sc.scratch[11].ptr, ok, n);
   if (rc) return rc;
-  and3_kernel<<<(unsigned)((n + 255) / 256), 256, 0, STREAM>>>((uint8_t*)ok, (const uint8_t*)sc.scratch[7].ptr,
-                                                             (const uint8_t*)sc.scratch[8].ptr, (long long)n);
-  CU(cudaGetLastError());
-  g_ctx.launches++;
-  return 0;
+  FlagList fl = {{(const uint8_t*)sc.scratch[7].ptr, (const uint8_t*)sc.scratch[8].ptr}, 2};
+  if (strict) {
+    rc = strict_flags_dev(sc.scratch[6].ptr, sc.scratch[11].ptr, n, fl);
+    if (rc) return rc;
+  }
+  return and_flags_dev(ok, fl, n);
 }
 
 // x bytes of each affine point with (flag << 7) OR-ed into byte 0 (bls_py/ec.py:103-111)
@@ -1356,6 +1413,27 @@ int b200bls_g2_compress_batch(const uint8_t* in, uint8_t* out, size_t n) {
   HostIO io[2] = {{in, nullptr, 192 * n}, {nullptr, out, 96 * n}};
   return with_staging(io, 2, [&](void** d) { return compress_dev(true, d[0], d[1], n); });
 }
+int b200bls_subgroup_check_batch(int g2, const uint8_t* pts, uint8_t* ok, size_t n) {
+  std::lock_guard<std::mutex> lk(g_mu);
+  if (!pts || !ok) return fail(B200BLS_E_ARG, "null buffer");
+  size_t w = g2 ? 192 : 96;
+  HostIO io[2] = {{pts, nullptr, w * n}, {nullptr, ok, n}};
+  return with_staging(io, 2, [&](void** d) { return subgroup_check_dev(g2 != 0, d[0], d[1], n); });
+}
+int b200bls_subgroup_check_batch_dev(int g2, const void* pts, void* ok, size_t n) {
+  std::lock_guard<std::mutex> lk(g_mu);
+  return subgroup_check_dev(g2 != 0, pts, ok, n);
+}
+int b200bls_key_validate_batch(const uint8_t* pts, uint8_t* ok, size_t n) {
+  std::lock_guard<std::mutex> lk(g_mu);
+  if (!pts || !ok) return fail(B200BLS_E_ARG, "null buffer");
+  HostIO io[2] = {{pts, nullptr, 96 * n}, {nullptr, ok, n}};
+  return with_staging(io, 2, [&](void** d) { return point_flags_dev("g1_keyvalidate", false, d[0], d[1], n); });
+}
+int b200bls_key_validate_batch_dev(const void* pts, void* ok, size_t n) {
+  std::lock_guard<std::mutex> lk(g_mu);
+  return point_flags_dev("g1_keyvalidate", false, pts, ok, n);
+}
 
 // ---- hashing, multi-pairing, verification ----------------------------------------------------
 int b200bls_hash_to_g2_batch(const uint8_t* hashes, uint8_t* out, size_t n) {
@@ -1451,6 +1529,27 @@ int b200bls_verify_batch_wire(const uint8_t* pk48, const uint8_t* mh, const uint
 int b200bls_verify_batch_wire_dev(const void* pk48, const void* mh, const void* sig96, void* ok, size_t n) {
   std::lock_guard<std::mutex> lk(g_mu);
   return verify_wire_dev(pk48, mh, sig96, ok, n);
+}
+int b200bls_verify_batch_strict(const uint8_t* pk, const uint8_t* mh, const uint8_t* sig, uint8_t* ok, size_t n) {
+  std::lock_guard<std::mutex> lk(g_mu);
+  if (!pk || !mh || !sig || !ok) return fail(B200BLS_E_ARG, "null buffer");
+  HostIO io[4] = {{pk, nullptr, 96 * n}, {mh, nullptr, 32 * n}, {sig, nullptr, 192 * n}, {nullptr, ok, n}};
+  return with_staging(io, 4, [&](void** d) { return verify_strict_dev(d[0], d[1], d[2], d[3], n); });
+}
+int b200bls_verify_batch_strict_dev(const void* pk, const void* mh, const void* sig, void* ok, size_t n) {
+  std::lock_guard<std::mutex> lk(g_mu);
+  return verify_strict_dev(pk, mh, sig, ok, n);
+}
+int b200bls_verify_batch_wire_strict(const uint8_t* pk48, const uint8_t* mh, const uint8_t* sig96, uint8_t* ok,
+                                     size_t n) {
+  std::lock_guard<std::mutex> lk(g_mu);
+  if (!pk48 || !mh || !sig96 || !ok) return fail(B200BLS_E_ARG, "null buffer");
+  HostIO io[4] = {{pk48, nullptr, 48 * n}, {mh, nullptr, 32 * n}, {sig96, nullptr, 96 * n}, {nullptr, ok, n}};
+  return with_staging(io, 4, [&](void** d) { return verify_wire_dev(d[0], d[1], d[2], d[3], n, true); });
+}
+int b200bls_verify_batch_wire_strict_dev(const void* pk48, const void* mh, const void* sig96, void* ok, size_t n) {
+  std::lock_guard<std::mutex> lk(g_mu);
+  return verify_wire_dev(pk48, mh, sig96, ok, n, true);
 }
 
 namespace {
