@@ -372,6 +372,11 @@ bool fp_is_square(fp x) {
 // Bounds: for a < alpha q, b < beta q the result is < q (0.1016 alpha beta + 1): weakly
 // reduced inputs give < 1.41 q, sums of two (< 4q each) give < 2.63 q; intermediates stay
 // below (alpha + 1) q < 2^384 for alpha <= 8.  No final subtraction.
+// The limit is on the FIRST operand only: the second may be any 384-bit value (fp_to_mont passes
+// the raw input there, R^2 mod q first), but a first operand of 2^384 - 1 gives a wrong integer.
+// Every call site passes a first operand <= 4q: weakly reduced values, sums of two, R^2 mod q,
+// and in fp_inv a canonical r0.  tests/fp_exact.py models the exact integer and
+// tests/test_fp_bounds_cpu.py pins both sides of the limit.
 //
 // (Tried and rejected, measured on B200: separate 768-bit products + one Montgomery reduction
 // per Fq2 coefficient -- 744 instead of 900 limb products per Fq2 multiplication, but as many
@@ -707,7 +712,7 @@ FP_DEV void fp2_mul(fp2& r, const fp2& a, const fp2& b) {
   fp_mul(t0, a.c0, b.c0);
   fp_mul(t1, a.c1, b.c1);
   fp_mul(t2, sa, sb);
-  fp_cond_sub_2q(t2, t2);
+  fp_cond_sub_2q(t2, t2);  // keeps fp_sub's input < 2q; c1 = t2 - t0 - t1 < 1.81 q either way
   fp_sub(r.c0, t0, t1);
   fp_sub(t2, t2, t0);
   fp_sub(r.c1, t2, t1);
@@ -718,7 +723,7 @@ FP_DEV void fp2_sqr(fp2& r, const fp2& a) {
   fp_add_raw(s, a.c0, a.c1);        // < 4q
   fp_sub_raw_2q(d, a.c0, a.c1);     // in (0, 4q)
   fp_add_raw(e, a.c0, a.c0);        // < 4q
-  fp_mul(c0, s, d);                 // < 2.63 q
+  fp_mul(c0, s, d);                 // s d <= (a0 + q)^2 < 9 q^2: < 1.92 q, the subtraction below never fires
   fp_mul(r.c1, e, a.c1);            // < 1.82 q
   fp_cond_sub_2q(r.c0, c0);
 }

@@ -37,6 +37,25 @@ FP_DEV void fp_xi_coeff(fp& r, bool role, const fp& own, const fp& oth) {
   fp_add(r, own, t);  // own < 2q, t <= 2q
 }
 
+// coefficient `role` of (own + oth u)^2 for role 0 (own = a0) / role 1 (own = a1):
+// role 0: (a0 + a1)(a0 - a1 + 2q); role 1: (a1 + a1) a0 -- sums left unreduced (< 4q)
+FP_DEV void fp_sqr2_coeff(fp& z, bool role, const fp& own, const fp& oth) {
+  fp p, dd, x;
+  fp_select(x, role, own, oth);
+  fp_add_raw(p, own, x);
+  fp_sub_raw_2q(dd, own, oth);
+  fp_select(x, role, oth, dd);
+  fp_mul(z, p, x);
+  fp_cond_sub_2q(z, z);  // never fires: role 0 < 1.92 q ((a0 + a1)(a0 - a1 + 2q) <= (a0 + q)^2), role 1 < 1.82 q
+}
+
+// the second row's left operand of MUL2: role 0 computes a0 b0 + (2q - a1) b1, role 1 a1 b0 + a0 b1
+FP_DEV void fp_mul2_oth(fp& r, bool role, const fp& oth) {
+  fp n;
+  fp_neg_raw_2q(n, oth);
+  fp_select(r, role, oth, n);
+}
+
 template <class Env>
 FP_DEV int vm_exec2(Env& env, uint32_t w0, uint32_t w1) {
   const int op = w0 & 0xff;
@@ -57,22 +76,15 @@ FP_DEV int vm_exec2(Env& env, uint32_t w0, uint32_t w1) {
         else
           fp_sub(z, x, y);
       } else if (op == OP_SQR2) {
-        // role 0: (a0 + a1)(a0 - a1 + 2q); role 1: (a1 + a1) a0 -- sums left unreduced (< 4q)
-        fp own, oth, p, dd, x;
+        fp own, oth;
         env.ld_own(a >> 1, own);
         env.ld_oth(a >> 1, oth);
-        fp_select(x, role, own, oth);
-        fp_add_raw(p, own, x);
-        fp_sub_raw_2q(dd, own, oth);
-        fp_select(x, role, oth, dd);
-        fp_mul(z, p, x);
-        fp_cond_sub_2q(z, z);
+        fp_sqr2_coeff(z, role, own, oth);
       } else {
-        fp own, oth, n;
+        fp own, oth;
         env.ld_own(a >> 1, own);
         env.ld_oth(a >> 1, oth);
-        fp_neg_raw_2q(n, oth);
-        fp_select(oth, role, oth, n);
+        fp_mul2_oth(oth, role, oth);
         // role 0: own * b_own + (2q - oth) * b_oth; role 1: own * b_oth + oth * b_own
         env.mul2(z, own, oth, b >> 1, role);
       }

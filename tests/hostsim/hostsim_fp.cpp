@@ -1,35 +1,10 @@
-// Host build of csrc/fp.cuh with the PTX instructions emulated (carry flag included).
-// TEST INFRASTRUCTURE: lets the CPU-only box check the exact limb/carry sequences that the
-// GPU executes.  Never linked into the product library.
+// Host build of the Fq primitive probe (tests/fp_probe.cu) with the PTX instructions emulated (carry flag
+// included).  TEST INFRASTRUCTURE: lets the CPU-only box check the exact limb/carry sequences of csrc/fp.cuh,
+// vm_exec.cuh and vm_exec2.cuh against tests/fp_exact.py.  Never linked into the product library.
 #define B200BLS_HOSTSIM 1
-#include "../../python-bls_b200/csrc/fp.cuh"
-using namespace b200bls;
-extern "C" {
-void hs_fp_mul(const uint32_t* a, const uint32_t* b, uint32_t* r) {
-  fp x, y, z;
-  for (int i = 0; i < NL; i++) { x.v[i] = a[i]; y.v[i] = b[i]; }
-  fp_mul(z, x, y);
-  for (int i = 0; i < NL; i++) r[i] = z.v[i];
-}
-void hs_fp_op(int op, const uint32_t* a, const uint32_t* b, uint32_t* r) {
-  fp x, y, z;
-  for (int i = 0; i < NL; i++) { x.v[i] = a[i]; y.v[i] = b[i]; }
-  switch (op) {
-    case 0: fp_add(z, x, y); break;
-    case 1: fp_sub(z, x, y); break;
-    case 2: fp_neg(z, x); break;
-    case 3: fp_set_zero(z); z.v[0] = fp_raw_gt(x, y); break;
-  }
-  for (int i = 0; i < NL; i++) r[i] = z.v[i];
-}
-void hs_fp2_op(int op, const uint32_t* a, const uint32_t* b, uint32_t* r) {
-  fp2 x, y, z;
-  for (int i = 0; i < NL; i++) { x.c0.v[i] = a[i]; x.c1.v[i] = a[NL + i]; y.c0.v[i] = b[i]; y.c1.v[i] = b[NL + i]; }
-  switch (op) {
-    case 0: fp2_mul(z, x, y); break;
-    case 1: fp2_sqr(z, x); break;
-    case 2: fp2_mul_xi(z, x); break;
-  }
-  for (int i = 0; i < NL; i++) { r[i] = z.c0.v[i]; r[NL + i] = z.c1.v[i]; }
-}
+#include "../fp_probe.cu"
+
+extern "C" int hs_fp_probe_run(long long n, const int* ops, const uint32_t* in, uint32_t* out) {
+  for (long long i = 0; i < n; i++) b200bls::probe_one(ops[i], in + i * 4 * b200bls::NL, out + i * 2 * b200bls::NL);
+  return 0;
 }
