@@ -11,6 +11,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <initializer_list>
 #include <map>
 #include <mutex>
 #include <string>
@@ -21,6 +22,7 @@
 #include "sha256.cuh"
 #include "gen/vm_isa.h"
 #include "vm_launch.h"
+#include "vm_plan.h"
 
 using namespace b200bls;
 
@@ -51,20 +53,15 @@ int fail(int code, const char* fmt, ...) {
 
 struct BlobEntry {
   char name[32];
-  uint32_t n_ins, body_start, epi_start, n_consts, n_slots, n_cold, n_tmem, ctas;
+  uint32_t n_ins, body_start, epi_start, n_consts, n_slots, n_cold, n_tmem, shape;
   uint64_t code_off, consts_off;
 };
 static_assert(sizeof(BlobEntry) == 32 + 32 + 16, "blob entry layout");
 
-struct DevProgram {
+struct DevProgram : ProgramShape {
   uint2* code = nullptr;
   uint4* consts = nullptr;
-  int n_ins = 0, body_start = 0, epi_start = 0, n_slots = 0, n_cold = 0, n_tmem = 0, ctas = 1;
-  int threads = VM_NT;  // shape 4 ("wide"): one CTA of VM_NT_WIDE threads per SM
-  // paired kernel (vm_kernel2.cuh): two threads per item
-  int items = 128;            // items per CTA: 128 (256 threads, 1-3 CTAs per SM) or 192 (384 threads, 2 CTAs per SM)
-  int ctas2 = 1;              // CTAs per SM of the paired kernel
-  bool cross_thread = false;  // the program has block barriers / cross-thread reads: CTA-wide item blocks
+  int n_ins = 0, body_start = 0, epi_start = 0;
 };
 
 struct Staging {
@@ -72,10 +69,42 @@ struct Staging {
   size_t cap = 0;
 };
 
+// Per-stream device buffers of the host-pointer entry points and the multi-stage pipelines, grown on demand and
+// kept.  Names with the same value share one buffer: their pipelines never run inside one another.
+enum Buf {
+  HOST_IO = 0,   // with_staging: the device copy of host argument i is buffer HOST_IO + i (i < VM_MAX_BUFS)
+  // aggregate_miller_host: the aggregate entry points stage their inputs themselves, never inside with_staging
+  AGG_P = HOST_IO, AGG_MH, AGG_Q, AGG_MILLER, AGG_GIVEN,
+  GATHERED = HOST_IO + 5,   // gather_partials: all ranks' partials (host gather)
+  SHARD_ACC,                // sharded entry points: this rank's partial, then the combined result
+  // device pipelines, each of which may run inside the ones above
+  SUM_PARTS = HOST_IO + VM_MAX_BUFS,   // sum_dev: one partial per CTA
+  SUM_THREAD_PARTS,         // sum_dev in three passes: one partial per thread
+  MILLER_RAW,               // miller_product_dev, aggregate_miller_dev: one raw Miller value per item
+  PROD_PARTS,               // raw_product_dev (inside the two above): one partial product per CTA
+  SHA_OUT,                  // sha_stage_dev output: aggregate_miller_dev, hash_to_g2_dev, verify_dev
+  MSM_MONT,                 // msm_dev (calls sum_dev): the points in Montgomery limbs
+  MSM_SEG_SUMS,             //   segment sums (or the per-point products of a small MSM)
+  MSM_COUNT,                //   bucket counts / cursors
+  MSM_OFFSETS,              //   bucket offsets, segment counts
+  MSM_IDX,                  //   point indices grouped by bucket
+  MSM_SEGMENTS,             //   segment offsets and scalars
+  MSM_SCALED,               //   segment sums times their bucket scalars
+  // verify_wire_dev (calls verify_dev and strict_flags_dev) and msm_dev never run inside one another
+  WIRE_PK = MSM_SEG_SUMS,   // decoded keys
+  WIRE_PK_OK = MSM_COUNT,   // key decoding flags
+  WIRE_SIG_OK = MSM_OFFSETS,   // signature decoding flags
+  WIRE_SIG = MSM_SCALED,    // decoded signatures
+  STRICT_FLAGS,             // strict_flags_dev: key and signature subgroup flags
+  CFLAGS,                   // compress_dev: the flag bit of every point
+  MULTI_PRODUCT = CFLAGS,   // b200bls_pairing_multi_dev (calls miller_product_dev): the Miller product
+  N_BUFS
+};
+
 constexpr int N_STREAMS = 8;
 
 // Everything a launch needs privately, so that launches on different streams can overlap:
-// the spill (cold) area, the item-block counter and the multi-stage scratch buffers.
+// the spill (cold) area, the item-block counter and the multi-stage buffers.
 struct StreamCtx {
   cudaStream_t stream = nullptr;
   cudaEvent_t done = nullptr;
@@ -83,26 +112,18 @@ struct StreamCtx {
   size_t cold_bytes = 0;
   int* counters = nullptr;   // ring of item-block counters, one per launch in flight
   unsigned counter_pos = 0;
-  Staging scratch[14];       // device-side intermediates of multi-stage entry points
-  Staging staging[VM_MAX_BUFS];  // device copies of the caller's host buffers
+  Staging bufs[N_BUFS];
 };
 constexpr int N_COUNTERS = 256;
 
 struct Context {
   bool ready = false;
   int device = -1;
-  int sm_count = 0;
+  Policy policy;   // sm_count, B200BLS_KERNEL, b200bls_set_ctas_per_sm
   StreamCtx sc[N_STREAMS];
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   std::map<std::string, DevProgram> programs;
   uint64_t launches = 0;
-  int ctas_per_sm = 0;   // launch shape: CTAs of 128 threads per SM (programs/registry.py); 0 = auto
-  // 1 = one thread per item (vm_kernel.cuh: the throughput kernel, 1.7 M pairings/s on whole waves); 2 = two
-  // threads per item (vm_kernel2.cuh: 0.7x the throughput, but 0.7x the latency of a pass -- 14.0 instead of
-  // 20.0 ms for up to 9,472 pairings); 0 = choose per launch: the paired kernel for isolated batches that leave
-  // most of the GPU empty, the one-thread kernel otherwise.  Environment variable B200BLS_KERNEL.
-  int kernel = 0;
-  int isolated_shape = 0;   // experiments: B200BLS_ISOLATED_SHAPE forces the shape of automatic (isolated) launches
   // segment tables of the serial tiny sums (sum_dev): idx[16] = 0..15, then for n = 0..16 the pair {0, n}
   unsigned* tiny_seg = nullptr;
 };
@@ -117,11 +138,10 @@ thread_local int t_stream = 0;
 StreamCtx& cur() { return g_ctx.sc[t_stream]; }
 #define STREAM (cur().stream)
 
-int ensure_buf(Staging& s, size_t bytes);
-int ensure_staging(int i, size_t bytes) { return ensure_buf(cur().staging[i], bytes); }
-int ensure_scratch(int i, size_t bytes) { return ensure_buf(cur().scratch[i], bytes); }
+void* dbuf(Buf b) { return cur().bufs[b].ptr; }
 
-int ensure_buf(Staging& s, size_t bytes) {
+int ensure(Buf b, size_t bytes) {
+  Staging& s = cur().bufs[b];
   if (s.cap >= bytes) return 0;
   if (s.ptr) cudaFree(s.ptr);
   s.ptr = nullptr;
@@ -133,44 +153,26 @@ int ensure_buf(Staging& s, size_t bytes) {
   return 0;
 }
 
-// grid: ctas_per_sm CTAs per SM at most; fewer when the batch is small
 struct SegArgs {
   const unsigned* start;  // n_items + 1 offsets
   const unsigned* idx;
 };
 
-int launch_program2(const DevProgram& pr, size_t n_items, const VmBuf* bufs, int n_bufs, int grid_override,
-                    const SegArgs* seg);
-
 int launch_program(const DevProgram& pr, size_t n_items, const VmBuf* bufs, int n_bufs, int grid_override = 0,
                    const SegArgs* seg = nullptr) {
-  Context& c = g_ctx;
-  if (c.kernel == 2 && pr.ctas2 > 0) return launch_program2(pr, n_items, bufs, n_bufs, grid_override, seg);
-  // automatic: latency-bound launches (at most one 128-item block per SM, no block reduction) go to the paired kernel
-  if (c.kernel == 0 && c.ctas_per_sm == 0 && grid_override == 0 && !seg && !pr.cross_thread &&
-      n_items <= (size_t)c.sm_count * 128)
-    return launch_program2(pr, n_items, bufs, n_bufs, grid_override, seg);
-  const int nt = pr.threads;
-  if (seg) grid_override = (int)((n_items + nt - 1) / nt);  // one thread per segment, statically assigned
-  long long blocks_needed = (long long)((n_items + nt - 1) / nt);
-  long long max_grid = (long long)c.sm_count * pr.ctas;
-  int grid = (int)(blocks_needed < max_grid ? blocks_needed : max_grid);
-  if (grid < 1) grid = 1;
-  if (grid_override > 0) grid = grid_override;
-  // (sized for the largest grid of the shape: the warp-fetch policy below may spread a small batch over more CTAs)
-  long long total = (long long)(grid > max_grid ? grid : max_grid) * nt;
+  Plan pl;
+  int rc = plan_launch(g_ctx.policy, pr, n_items, grid_override, seg != nullptr, pl);
+  if (rc == B200BLS_E_ARG) return fail(rc, "%zu items exceed the paired kernel's 2^31 - 1", n_items);
+  if (rc) return fail(rc, "shape %d: %d TMEM slots do not fit its columns", pr.shape, pr.n_tmem);
   StreamCtx& sc = cur();
-  size_t cold_need = (size_t)pr.n_cold * 6 * sizeof(uint4) * total;
-  if (cold_need > sc.cold_bytes) {
+  if (pl.cold_bytes > sc.cold_bytes) {
     CU(cudaStreamSynchronize(sc.stream));
     if (sc.cold) cudaFree(sc.cold);
     sc.cold = nullptr;
     sc.cold_bytes = 0;
-    size_t want = (size_t)pr.n_cold * 6 * sizeof(uint4) * (size_t)max_grid * nt;
-    if (want < cold_need) want = cold_need;
-    cudaError_t e = cudaMalloc(&sc.cold, want);
-    if (e != cudaSuccess) return fail(B200BLS_E_NOMEM, "cold area cudaMalloc(%zu) failed", want);
-    sc.cold_bytes = want;
+    cudaError_t e = cudaMalloc(&sc.cold, pl.cold_bytes);
+    if (e != cudaSuccess) return fail(B200BLS_E_NOMEM, "cold area cudaMalloc(%zu) failed", pl.cold_bytes);
+    sc.cold_bytes = pl.cold_bytes;
   }
   int* counter = sc.counters + (sc.counter_pos++ % N_COUNTERS);
   CU(cudaMemsetAsync(counter, 0, sizeof(int), sc.stream));
@@ -183,213 +185,80 @@ int launch_program(const DevProgram& pr, size_t n_items, const VmBuf* bufs, int 
   p.consts = pr.consts;
   p.cold = sc.cold;
   p.n_items = (long long)n_items;
-  p.n_blocks = (long long)((n_items + nt - 1) / nt);
-  p.counter = counter;
-  if (seg) {
-    p.seg_start = seg->start;
-    p.seg_idx = seg->idx;
-  }
-  // (not for shape 5: with 16 warps per CTA some scheduler holds four warps whether the batch is spread or not, and
-  // CTA-wide blocks keep the warps of a CTA together in the program: 65,536 pairings 45.6 instead of 47.3 ms)
-  if (!pr.cross_thread && !seg && c.ctas_per_sm == 0 && grid_override == 0 && nt != VM_NT_XWIDE) {
-    // An isolated batch (automatic shape): item blocks of 32 per WARP, spread over all SMs, and when the batch
-    // is w.f waves long it runs as ceil(w.f) equal waves on fewer warps per CTA (a warp is faster at lower
-    // occupancy): 65,536 pairings = 1.15 waves took 33 + 32 ms, two passes at 7 of 12 warps take 52.  With an
-    // explicit shape (pipelines that keep launches in flight) blocks stay CTA-wide: the barrier per block keeps
-    // a CTA's warps near each other in the program, which the instruction cache rewards (33.1 vs 34.3 ms).
-    const int warps = nt / 32;
-    p.warp_fetch = 1;
-    p.n_blocks = (long long)((n_items + 31) / 32);
-    p.active_warps = warps;
-    {
-      const long long cap = max_grid * warps;
-      const long long waves = (p.n_blocks + cap - 1) / cap;
-      const long long per_wave = (p.n_blocks + waves - 1) / waves;
-      const int g2 = (int)(per_wave < max_grid ? per_wave : max_grid);
-      long long act = (per_wave + g2 - 1) / g2;
-      if (act < 1) act = 1;
-      if (act < warps) p.active_warps = (int)act;
-      if ((long long)g2 * nt <= total) grid = g2;   // never beyond what the cold area was sized for
-    }
-  }
-  p.smem_cells = 2 * pr.n_slots;
-  for (int i = 0; i < n_bufs && i < VM_MAX_BUFS; i++) p.bufs[i] = bufs[i];
-  size_t smem = (size_t)pr.n_slots * 2 * 3 * sizeof(uint4) * nt;
-  if (nt == VM_NT_XWIDE) {
-    // four groups of four warps: 128 columns each (5 Fq2 slots)
-    if (pr.n_tmem * 24 > 128) return fail(B200BLS_E_PROGRAM, "shape 5: %d TMEM slots do not fit 128 columns", pr.n_tmem);
-    p.tmem_cols = 512;
-    p.tmem_group_cols = 128;
-    vm3_launch(grid, smem, sc.stream, p);
-  } else if (nt == VM_NT_WIDE) {
-    // three groups of four warps share the SM's 512 columns: 168 each (7 Fq2 slots)
-    if (pr.n_tmem * 24 > 168) return fail(B200BLS_E_PROGRAM, "wide shape: %d TMEM slots do not fit 168 columns", pr.n_tmem);
-    p.tmem_cols = 512;
-    p.tmem_group_cols = 168;
-    vm1_launch(true, true, grid, smem, sc.stream, p);
-  } else {
-    p.tmem_cols = pr.n_tmem == 0 ? 0 : (pr.n_tmem * 24 <= 128 ? 128 : (pr.n_tmem * 24 <= 256 ? 256 : 512));
-    p.tmem_group_cols = 0;
-    vm1_launch(p.tmem_cols != 0, false, grid, smem, sc.stream, p);
-  }
-  CU(cudaGetLastError());
-  c.launches++;
-  return 0;
-}
-
-// The paired kernel: two threads per item.  Per-item resources (slots, TMEM columns, cold slots) are
-// those the program was assembled for; a CTA holds pr.items items on 2 * pr.items threads.
-int launch_program2(const DevProgram& pr, size_t n_items, const VmBuf* bufs, int n_bufs, int grid_override,
-                    const SegArgs* seg) {
-  Context& c = g_ctx;
-  const int items = pr.items, nt = 2 * items;
-  const long long cta_blocks = (long long)((n_items + items - 1) / items);
-  const long long max_grid = (long long)c.sm_count * pr.ctas2;
-  int grid = (int)(cta_blocks < max_grid ? cta_blocks : max_grid);
-  if (grid < 1) grid = 1;
-  if (seg) grid_override = (int)cta_blocks;  // one pair per segment, statically assigned
-  if (grid_override > 0) grid = grid_override;
-  StreamCtx& sc = cur();
-  // the cold area is sized for the largest grid of this shape: the warp-fetch policy below may raise `grid`
-  const long long total = (long long)(grid > max_grid ? grid : max_grid) * nt;  // threads
-  const size_t cold_need = (size_t)pr.n_cold * 3 * sizeof(uint4) * total;
-  if (cold_need > sc.cold_bytes) {
-    CU(cudaStreamSynchronize(sc.stream));
-    if (sc.cold) cudaFree(sc.cold);
-    sc.cold = nullptr;
-    sc.cold_bytes = 0;
-    size_t want = (size_t)pr.n_cold * 3 * sizeof(uint4) * (size_t)max_grid * nt;
-    if (want < cold_need) want = cold_need;
-    cudaError_t e = cudaMalloc(&sc.cold, want);
-    if (e != cudaSuccess) return fail(B200BLS_E_NOMEM, "cold area cudaMalloc(%zu) failed", want);
-    sc.cold_bytes = want;
-  }
-  int* counter = sc.counters + (sc.counter_pos++ % N_COUNTERS);
-  CU(cudaMemsetAsync(counter, 0, sizeof(int), sc.stream));
-  VmParams p;
-  memset(&p, 0, sizeof(p));
-  p.code = pr.code;
-  p.body_start = pr.body_start;
-  p.epi_start = pr.epi_start;
-  p.n_ins = pr.n_ins;
-  p.consts = pr.consts;
-  p.cold = sc.cold;
-  p.n_items = (long long)n_items;
+  p.n_blocks = pl.n_blocks;
   p.counter = counter;
   if (seg) {
     p.seg_start = seg->start;
     p.seg_idx = seg->idx;
   }
   p.smem_cells = 2 * pr.n_slots;
-  const int warps = nt / 32;
-  if (!pr.cross_thread && !seg) {
-    // item blocks of 16 per warp.  An isolated batch (automatic shape) is spread over ALL SMs and, when it is
-    // w.f waves long, runs as ceil(w.f) EQUAL waves on fewer warps per CTA: a warp is faster at lower
-    // occupancy, so neither a partly filled last wave nor a handful of full CTAs on a few SMs is left.
-    p.warp_fetch = 1;
-    p.n_blocks = (long long)((n_items + VM2_ITEMS_PER_WARP - 1) / VM2_ITEMS_PER_WARP);
-    p.active_warps = warps;
-    if (c.ctas_per_sm == 0 && grid_override == 0) {
-      const long long cap = max_grid * warps;
-      const long long waves = (p.n_blocks + cap - 1) / cap;
-      const long long per_wave = (p.n_blocks + waves - 1) / waves;      // warps busy at a time
-      grid = (int)(per_wave < max_grid ? per_wave : max_grid);
-      long long act = (per_wave + grid - 1) / grid;
-      if (act < 1) act = 1;
-      if (act < warps) p.active_warps = (int)act;
-    }
-  } else {
-    p.n_blocks = cta_blocks;
-    p.active_warps = warps;
-  }
+  p.tmem_cols = pl.tmem_cols;
+  p.tmem_group_cols = pl.tmem_group_cols;
+  p.warp_fetch = pl.warp_fetch;
+  p.active_warps = pl.active_warps;
   for (int i = 0; i < n_bufs && i < VM_MAX_BUFS; i++) p.bufs[i] = bufs[i];
-  const size_t smem = (size_t)pr.n_slots * 3 * sizeof(uint4) * nt;
-  const int groups = nt / 128;
-  p.tmem_group_cols = pr.n_tmem * 12;
-  const int cols = groups * p.tmem_group_cols;
-  p.tmem_cols = cols == 0 ? 0 : (cols <= 128 ? 128 : (cols <= 256 ? 256 : 512));
-  if (cols > 512) return fail(B200BLS_E_PROGRAM, "%d TMEM slots do not fit 512 columns", pr.n_tmem);
-  vm2_launch(p.tmem_cols != 0, nt == VM2_NT_WIDE, seg != nullptr, grid, smem, sc.stream, p);
+  if (pl.family == 2)
+    vm2_launch(pl.use_tmem, pl.wide, pl.seg, pl.grid, pl.smem, sc.stream, p);
+  else if (pl.family == 3)
+    vm3_launch(pl.grid, pl.smem, sc.stream, p);
+  else
+    vm1_launch(pl.use_tmem, pl.wide, pl.grid, pl.smem, sc.stream, p);
   CU(cudaGetLastError());
-  c.launches++;
+  g_ctx.launches++;
   return 0;
 }
 
-// Auto shape for an isolated batch of n items: more CTAs per SM raise throughput but also the
-// latency of one pass (measured pairing pass: 1 : 1.3 : 1.85 for 1 : 2 : 3 CTAs/SM), so the best
-// shape minimises passes x latency.  Pipelines that keep several batches in flight (bench.py)
-// select the wide shape (4) explicitly.
-int auto_ctas(size_t n) {
-  static const double kLat[4] = {0, 1.0, 1.3, 1.85};
-  int best = 1;
-  double best_cost = 1e300;
-  for (int c = 1; c <= 3; c++) {
-    size_t cap = (size_t)g_ctx.sm_count * VM_NT * c;
-    double cost = (double)((n + cap - 1) / cap) * kLat[c];
-    if (cost < best_cost - 1e-9) {
-      best_cost = cost;
-      best = c;
-    }
-  }
-  return best;
-}
-
+// "<name>@<shape>": that program; "<name>": the shape choose_shape picks for n_items among those it was assembled for
 const DevProgram* find_program(const char* base, size_t n_items = 0) {
-  // "<name>@<ctas>": the configured shape, else the nearest one with fewer CTAs per SM
   std::string name(base);
-  if (name.find('@') != std::string::npos) {
-    auto it = g_ctx.programs.find(name);
-    if (it != g_ctx.programs.end()) return &it->second;
-  } else {
-    int want = g_ctx.ctas_per_sm > 0 ? g_ctx.ctas_per_sm : auto_ctas(n_items ? n_items : 1);
-    // the wide shape (id 4) holds as many items per SM as three narrow CTAs and is faster where it exists
-    if (g_ctx.ctas_per_sm == 0 && want == 3) want = 4;
-    if (g_ctx.ctas_per_sm == 0 && g_ctx.kernel != 2) {
-      // an isolated batch that is a little more than whole 384-item waves: fewer passes on the 512-thread shape
-      const size_t sm = (size_t)g_ctx.sm_count, n = n_items ? n_items : 1;
-      const size_t p16 = (n + sm * VM_NT_XWIDE - 1) / (sm * VM_NT_XWIDE), p12 = (n + sm * VM_NT_WIDE - 1) / (sm * VM_NT_WIDE);
-      if (n > sm * VM_NT && p16 < p12) want = 5;
-      if (g_ctx.isolated_shape > 0 && n > sm * VM_NT) want = g_ctx.isolated_shape;
-    }
-    if (want == 5 && g_ctx.kernel == 2) want = 4;   // the paired kernel has no 512-thread shape
-    for (int c = want; c >= 1; c--) {
-      auto it = g_ctx.programs.find(name + "@" + std::to_string(c));
-      if (it != g_ctx.programs.end()) return &it->second;
-    }
+  if (name.find('@') == std::string::npos) {
+    unsigned have = 0;
+    for (int s = 1; s <= N_SHAPES; s++)
+      if (g_ctx.programs.count(name + "@" + std::to_string(s))) have |= 1u << s;
+    if (int s = choose_shape(g_ctx.policy, n_items, have)) name += "@" + std::to_string(s);
   }
+  auto it = g_ctx.programs.find(name);
+  if (it != g_ctx.programs.end()) return &it->second;
   fail(B200BLS_E_PROGRAM, "unknown program '%s'", base);
   return nullptr;
 }
 
-struct HostBuf {
+// Every compute entry point runs under the library mutex, after its own argument checks, and only once
+// b200bls_init() has succeeded: there is no CPU path.
+template <class F>
+int locked(F&& body) {
+  std::lock_guard<std::mutex> lk(g_mu);
+  if (!g_ctx.ready) return fail(B200BLS_E_NOT_INIT, "b200bls_init() has not succeeded");
+  return body();
+}
+
+struct HostIO {
   const void* in;   // host source (nullptr for pure outputs)
   void* out;        // host destination (nullptr for pure inputs)
-  size_t stride;    // bytes per item
+  size_t bytes;
 };
 
-// copy inputs up, run, copy outputs back on the selected stream; synchronise unless the caller
-// asked for the asynchronous form (then b200bls_sync() must precede any use of the outputs and
-// the host buffers should be pinned so that the copies really overlap other streams' kernels)
-int run_host(const char* name, size_t n, const HostBuf* hb, int n_bufs, bool sync = true) {
-  if (!g_ctx.ready) return fail(B200BLS_E_NOT_INIT, "b200bls_init() has not succeeded");
-  const DevProgram* pr = find_program(name, n);
-  if (!pr) return B200BLS_E_PROGRAM;
-  if (n == 0) return 0;
-  VmBuf bufs[VM_MAX_BUFS];
-  memset(bufs, 0, sizeof(bufs));
-  for (int i = 0; i < n_bufs; i++) {
-    int rc = ensure_staging(i, hb[i].stride * n);
+// The host-pointer form of a device pipeline: copies the inputs up into buffers HOST_IO + i, runs body on the device
+// pointers and copies the outputs back on the calling thread's stream.  Synchronises unless async: then
+// b200bls_sync() must precede any use of the outputs, and pinned host buffers let the copies overlap other streams'
+// kernels.
+template <class F>
+int with_staging(const HostIO* io, int n_io, F&& body, bool async = false) {
+  return locked([&] {
+    void* dev[VM_MAX_BUFS];
+    for (int i = 0; i < n_io; i++) {
+      int rc = ensure(Buf(HOST_IO + i), io[i].bytes ? io[i].bytes : 1);
+      if (rc) return rc;
+      dev[i] = dbuf(Buf(HOST_IO + i));
+      if (io[i].in && io[i].bytes) CU(cudaMemcpyAsync(dev[i], io[i].in, io[i].bytes, cudaMemcpyHostToDevice, STREAM));
+    }
+    int rc = body(dev);
     if (rc) return rc;
-    bufs[i].ptr = (unsigned char*)cur().staging[i].ptr;
-    bufs[i].stride = (long long)hb[i].stride;
-    if (hb[i].in) CU(cudaMemcpyAsync(bufs[i].ptr, hb[i].in, hb[i].stride * n, cudaMemcpyHostToDevice, STREAM));
-  }
-  int rc = launch_program(*pr, n, bufs, n_bufs);
-  if (rc) return rc;
-  for (int i = 0; i < n_bufs; i++)
-    if (hb[i].out) CU(cudaMemcpyAsync(hb[i].out, bufs[i].ptr, hb[i].stride * n, cudaMemcpyDeviceToHost, STREAM));
-  if (sync) CU(cudaStreamSynchronize(STREAM));
-  return 0;
+    for (int i = 0; i < n_io; i++)
+      if (io[i].out && io[i].bytes) CU(cudaMemcpyAsync(io[i].out, dev[i], io[i].bytes, cudaMemcpyDeviceToHost, STREAM));
+    if (!async) CU(cudaStreamSynchronize(STREAM));
+    return 0;
+  });
 }
 
 struct DevBuf {
@@ -398,7 +267,6 @@ struct DevBuf {
 };
 
 int run_dev(const char* name, size_t n, const DevBuf* db, int n_bufs) {
-  if (!g_ctx.ready) return fail(B200BLS_E_NOT_INIT, "b200bls_init() has not succeeded");
   const DevProgram* pr = find_program(name, n);
   if (!pr) return B200BLS_E_PROGRAM;
   if (n == 0) return 0;
@@ -411,24 +279,33 @@ int run_dev(const char* name, size_t n, const DevBuf* db, int n_bufs) {
   return launch_program(*pr, n, bufs, n_bufs);
 }
 
-
-int grid_for(const DevProgram& pr, size_t n_items) {
-  const int per_cta = g_ctx.kernel == 2 ? pr.items : pr.threads;
-  long long blocks_needed = (long long)((n_items + per_cta - 1) / per_cta);
-  long long max_grid = (long long)g_ctx.sm_count * (g_ctx.kernel == 2 ? pr.ctas2 : pr.ctas);
-  long long g = blocks_needed < max_grid ? blocks_needed : max_grid;
-  return g < 1 ? 1 : (int)g;
+// one program on host buffers: io[i].bytes is the size of ONE item of argument i
+int run_host(const char* name, size_t n, std::initializer_list<HostIO> per_item, bool async = false) {
+  HostIO io[VM_MAX_BUFS];
+  DevBuf db[VM_MAX_BUFS];
+  const int k = (int)per_item.size();
+  for (int i = 0; i < k; i++) {
+    io[i] = per_item.begin()[i];
+    db[i].stride = io[i].bytes;
+    io[i].bytes *= n;
+  }
+  return with_staging(io, k, [&](void** d) {
+    for (int i = 0; i < k; i++) db[i].ptr = d[i];
+    return run_dev(name, n, db, k);
+  }, async);
 }
-
-#define NEED_READY()                                                                       \
-  do {                                                                                     \
-    if (!g_ctx.ready) return fail(B200BLS_E_NOT_INIT, "b200bls_init() has not succeeded"); \
-  } while (0)
 
 int launch_named(const char* name, size_t n, const VmBuf* bufs, int n_bufs, int grid_override = 0) {
   const DevProgram* pr = find_program(name, n);
   if (!pr) return B200BLS_E_PROGRAM;
   return launch_program(*pr, n, bufs, n_bufs, grid_override);
+}
+
+// the grid of a launch without override: block reductions size their per-CTA partials with it and fix it
+int grid_of(const DevProgram& pr, size_t n_items) {
+  Plan pl;
+  plan_launch(g_ctx.policy, pr, n_items, 0, false, pl);
+  return pl.grid;
 }
 
 VmBuf vb(const void* p, long long stride) {
@@ -447,7 +324,6 @@ constexpr size_t kSumOnePassMax = 1024;
 // Up to 6 points: one thread adds them one after the other (measured below that: 7 tree levels cost more).
 constexpr size_t kSumSerialMax = 6;
 int sum_dev(bool g2, const void* pts, void* out, size_t n) {
-  NEED_READY();
   const char* n1 = g2 ? "g2_sum1" : "g1_sum1";
   const char* n2 = g2 ? "g2_sum2" : "g1_sum2";
   size_t w = g2 ? 192 : 96;
@@ -466,41 +342,42 @@ int sum_dev(bool g2, const void* pts, void* out, size_t n) {
     VmBuf bs[2] = {vb(pts, (long long)w), vb(out, (long long)w)};
     return launch_named(g2 ? "g2_sums" : "g1_sums", n, bs, 2, 1);
   }
-  if (n >= kSumThreePassMin && g_ctx.kernel != 2) {
+  if (n >= kSumThreePassMin && g_ctx.policy.kernel != 2) {
     // Large sums in three passes.  A: every thread of the 12-warp shape folds its share with mixed additions and
     // stores its Jacobian partial (g?_sumf has no cross-thread step, so it is not held to two 128-thread CTAs per
     // SM like g?_sum1 with its tree); B: the partials are folded and tree-reduced per CTA (g?_sum1j); C: one CTA.
     const DevProgram* pf = find_program(g2 ? "g2_sumf@4" : "g1_sumf@4", n);
-    const DevProgram* pj = pf ? find_program(g2 ? "g2_sum1j" : "g1_sum1j", (size_t)g_ctx.sm_count * pf->threads) : nullptr;
+    const int nt = pf ? kShapes[pf->shape].threads : 0;
+    const DevProgram* pj = pf ? find_program(g2 ? "g2_sum1j" : "g1_sum1j", (size_t)g_ctx.policy.sm_count * nt) : nullptr;
     if (pf && pj) {
-      const int grid_a = grid_for(*pf, n);
-      const size_t parts = (size_t)grid_a * pf->threads;   // n >= parts: every thread is active in the epilogue
+      const int grid_a = grid_of(*pf, n);
+      const size_t parts = (size_t)grid_a * nt;   // n >= parts: every thread is active in the epilogue
       const size_t elems = g2 ? 3 : 2;
-      int rc = ensure_scratch(12, elems * 6 * sizeof(uint4) * parts);
+      int rc = ensure(SUM_THREAD_PARTS, elems * 6 * sizeof(uint4) * parts);
       if (rc) return rc;
-      VmBuf ba[2] = {vb(pts, (long long)w), vb(cur().scratch[12].ptr, (long long)parts)};
+      VmBuf ba[2] = {vb(pts, (long long)w), vb(dbuf(SUM_THREAD_PARTS), (long long)parts)};
       rc = launch_program(*pf, n, ba, 2, grid_a);
       if (rc) return rc;
-      const int grid_b = grid_for(*pj, parts);
-      rc = ensure_scratch(0, elems * 6 * sizeof(uint4) * grid_b);
+      const int grid_b = grid_of(*pj, parts);
+      rc = ensure(SUM_PARTS, elems * 6 * sizeof(uint4) * grid_b);
       if (rc) return rc;
-      VmBuf bb[2] = {vb(cur().scratch[12].ptr, (long long)parts), vb(cur().scratch[0].ptr, grid_b)};
+      VmBuf bb[2] = {vb(dbuf(SUM_THREAD_PARTS), (long long)parts), vb(dbuf(SUM_PARTS), grid_b)};
       rc = launch_program(*pj, parts, bb, 2, grid_b);
       if (rc) return rc;
-      VmBuf bc[2] = {vb(cur().scratch[0].ptr, grid_b), vb(out, (long long)w)};
+      VmBuf bc[2] = {vb(dbuf(SUM_PARTS), grid_b), vb(out, (long long)w)};
       return launch_named(n2, (size_t)grid_b, bc, 2, 1);
     }
   }
   const DevProgram* p1 = find_program(n1, n);
   if (!p1) return B200BLS_E_PROGRAM;
-  int grid = grid_for(*p1, n);
+  int grid = grid_of(*p1, n);
   size_t raw_bytes = (size_t)(g2 ? 3 : 2) * 6 * sizeof(uint4) * grid;
-  int rc = ensure_scratch(0, raw_bytes);
+  int rc = ensure(SUM_PARTS, raw_bytes);
   if (rc) return rc;
-  VmBuf b1[2] = {vb(pts, (long long)w), vb(cur().scratch[0].ptr, grid)};
+  VmBuf b1[2] = {vb(pts, (long long)w), vb(dbuf(SUM_PARTS), grid)};
   rc = launch_program(*p1, n, b1, 2, grid);
   if (rc) return rc;
-  VmBuf b2[2] = {vb(cur().scratch[0].ptr, grid), vb(out, (long long)w)};
+  VmBuf b2[2] = {vb(dbuf(SUM_PARTS), grid), vb(out, (long long)w)};
   return launch_named(n2, (size_t)grid, b2, 2, 1);
 }
 
@@ -611,18 +488,17 @@ __global__ void msm_scatter_kernel(const uint8_t* __restrict__ scalars, const un
 }
 
 int msm_dev(bool g2, const void* pts, const void* scalars, void* out, size_t n) {
-  NEED_READY();
   const size_t w = g2 ? 192 : 96;
   const char* mul = g2 ? "g2_mul" : "g1_mul";
   if (n >= 0xffffffffull / MSM_W) return fail(B200BLS_E_ARG, "msm: too many points");
   if (n < MSM_MIN_N) {  // per-point ladder, then the reduction
     if (n == 0) return sum_dev(g2, pts, out, 0);
-    int rc = ensure_scratch(6, w * n);
+    int rc = ensure(MSM_SEG_SUMS, w * n);
     if (rc) return rc;
-    VmBuf b[3] = {vb(pts, (long long)w), vb(scalars, 32), vb(cur().scratch[6].ptr, (long long)w)};
+    VmBuf b[3] = {vb(pts, (long long)w), vb(scalars, 32), vb(dbuf(MSM_SEG_SUMS), (long long)w)};
     rc = launch_named(mul, n, b, 3);
     if (rc) return rc;
-    return sum_dev(g2, cur().scratch[6].ptr, out, n);
+    return sum_dev(g2, dbuf(MSM_SEG_SUMS), out, n);
   }
   // longest run one thread folds: the mean bucket size plus seven standard deviations, so that
   // uniformly distributed digits are never cut and skewed ones are spread over many threads
@@ -630,19 +506,19 @@ int msm_dev(bool g2, const void* pts, const void* scalars, void* out, size_t n) 
   const unsigned seg_len = (unsigned)(mean + 7.0 * sqrt(mean) + 16.0);
   const long long pairs = (long long)n * MSM_W;
   const size_t seg_cap = (size_t)MSM_B + (size_t)(pairs / seg_len) + 1;     // upper bound on the number of segments
-  int rc = ensure_scratch(6, w * seg_cap);                                  // segment sums
-  if (!rc) rc = ensure_scratch(7, sizeof(unsigned) * (size_t)MSM_B);        // counts / cursors
-  if (!rc) rc = ensure_scratch(8, sizeof(unsigned) * 2 * ((size_t)MSM_B + 1));  // bucket offsets, segment counts
-  if (!rc) rc = ensure_scratch(9, sizeof(unsigned) * (size_t)pairs);        // point indices grouped by bucket
-  if (!rc) rc = ensure_scratch(10, (size_t)36 * (seg_cap + 1));             // segment offsets + scalars
-  if (!rc) rc = ensure_scratch(11, w * seg_cap);                            // segment sums times bucket scalars
+  int rc = ensure(MSM_SEG_SUMS, w * seg_cap);                                  // segment sums
+  if (!rc) rc = ensure(MSM_COUNT, sizeof(unsigned) * (size_t)MSM_B);        // counts / cursors
+  if (!rc) rc = ensure(MSM_OFFSETS, sizeof(unsigned) * 2 * ((size_t)MSM_B + 1));  // bucket offsets, segment counts
+  if (!rc) rc = ensure(MSM_IDX, sizeof(unsigned) * (size_t)pairs);        // point indices grouped by bucket
+  if (!rc) rc = ensure(MSM_SEGMENTS, (size_t)36 * (seg_cap + 1));             // segment offsets + scalars
+  if (!rc) rc = ensure(MSM_SCALED, w * seg_cap);                            // segment sums times bucket scalars
   if (rc) return rc;
   StreamCtx& sc = cur();
-  unsigned* count = (unsigned*)sc.scratch[7].ptr;
-  unsigned* start = (unsigned*)sc.scratch[8].ptr;
+  unsigned* count = (unsigned*)dbuf(MSM_COUNT);
+  unsigned* start = (unsigned*)dbuf(MSM_OFFSETS);
   unsigned* seg_first = start + MSM_B + 1;
-  unsigned* idx = (unsigned*)sc.scratch[9].ptr;
-  unsigned* seg_start = (unsigned*)sc.scratch[10].ptr;
+  unsigned* idx = (unsigned*)dbuf(MSM_IDX);
+  unsigned* seg_start = (unsigned*)dbuf(MSM_SEGMENTS);
   uint8_t* seg_scalar = (uint8_t*)(seg_start + ((seg_cap + 1 + 7) & ~(size_t)7));
   const unsigned pair_grid = (unsigned)((pairs + 255) / 256);
   CU(cudaMemsetAsync(count, 0, sizeof(unsigned) * MSM_B, STREAM));
@@ -658,54 +534,65 @@ int msm_dev(bool g2, const void* pts, const void* scalars, void* out, size_t n) 
   if (n_seg == 0) return sum_dev(g2, pts, out, 0);  // every scalar is zero
   if (n_seg > seg_cap) return fail(B200BLS_E_CUDA, "msm: segment count %u exceeds its bound %zu", n_seg, seg_cap);
   // every point is read once per window: convert it to Montgomery limbs once (SoA copy), not MSM_W times in the fold
-  rc = ensure_scratch(4, w * n);
+  rc = ensure(MSM_MONT, w * n);
   if (rc) return rc;
-  VmBuf bt[2] = {vb(pts, (long long)w), vb(sc.scratch[4].ptr, (long long)n)};
+  VmBuf bt[2] = {vb(pts, (long long)w), vb(dbuf(MSM_MONT), (long long)n)};
   rc = launch_named(g2 ? "g2_tomont" : "g1_tomont", n, bt, 2);
   if (rc) return rc;
   const DevProgram* fold = find_program(g2 ? "g2_bucketr" : "g1_bucketr", n_seg);
   if (!fold) return B200BLS_E_PROGRAM;
   SegArgs seg = {seg_start, idx};
-  VmBuf bf[2] = {vb(sc.scratch[4].ptr, (long long)n), vb(sc.scratch[6].ptr, (long long)w)};
+  VmBuf bf[2] = {vb(dbuf(MSM_MONT), (long long)n), vb(dbuf(MSM_SEG_SUMS), (long long)w)};
   rc = launch_program(*fold, n_seg, bf, 2, 0, &seg);
   if (rc) return rc;
-  VmBuf bm[3] = {vb(sc.scratch[6].ptr, (long long)w), vb(seg_scalar, 32), vb(sc.scratch[11].ptr, (long long)w)};
+  VmBuf bm[3] = {vb(dbuf(MSM_SEG_SUMS), (long long)w), vb(seg_scalar, 32), vb(dbuf(MSM_SCALED), (long long)w)};
   rc = launch_named(g2 ? "g2_bscale" : "g1_bscale", n_seg, bm, 3);
   if (rc) return rc;
-  return sum_dev(g2, sc.scratch[11].ptr, out, n_seg);
+  return sum_dev(g2, dbuf(MSM_SCALED), out, n_seg);
 }
 
 // ---- multi-pairing: Miller loops -> raw Fq12 per item -> product tree ------------------------
 // out576: big-endian product of the Miller values (not final-exponentiated)
-// product of the n raw Miller values in scratch[1] -> out576 (big-endian, not final-exponentiated)
+// product of the n raw Miller values in buffer MILLER_RAW -> out576 (big-endian, not final-exponentiated)
 int raw_product_dev(void* out576, size_t n) {
   const DevProgram* p1 = find_program("f12_prod1", n);
   if (!p1) return B200BLS_E_PROGRAM;
-  int grid = grid_for(*p1, n);
-  int rc = ensure_scratch(2, (size_t)576 * grid);
+  int grid = grid_of(*p1, n);
+  int rc = ensure(PROD_PARTS, (size_t)576 * grid);
   if (rc) return rc;
-  VmBuf bb[2] = {vb(cur().scratch[1].ptr, (long long)n), vb(cur().scratch[2].ptr, grid)};
+  VmBuf bb[2] = {vb(dbuf(MILLER_RAW), (long long)n), vb(dbuf(PROD_PARTS), grid)};
   rc = launch_program(*p1, n, bb, 2, grid);
   if (rc) return rc;
-  VmBuf bc[2] = {vb(cur().scratch[2].ptr, grid), vb(out576, 576)};
+  VmBuf bc[2] = {vb(dbuf(PROD_PARTS), grid), vb(out576, 576)};
   return launch_named("f12_prod2", (size_t)grid, bc, 2, 1);
 }
 
+// the Fq12 one (big-endian) -> out576: the empty product
+int fq12_one_dev(void* out576) {
+  static const uint8_t kOne[48] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0,
+                                   0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 1};
+  CU(cudaMemsetAsync(out576, 0, 576, STREAM));
+  CU(cudaMemcpyAsync(out576, kOne, 48, cudaMemcpyHostToDevice, STREAM));
+  return 0;
+}
+
 int miller_product_dev(const void* P, const void* Q, void* out576, size_t n) {
-  NEED_READY();
-  if (n == 0) {  // the empty product (fields_t.py:1117: prod starts at one)
-    static const uint8_t kOne[48] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0,
-                                     0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 1};
-    CU(cudaMemsetAsync(out576, 0, 576, STREAM));
-    CU(cudaMemcpyAsync(out576, kOne, 48, cudaMemcpyHostToDevice, STREAM));
-    return 0;
-  }
-  int rc = ensure_scratch(1, (size_t)576 * n);
+  if (n == 0) return fq12_one_dev(out576);   // fields_t.py:1117: prod starts at one
+  int rc = ensure(MILLER_RAW, (size_t)576 * n);
   if (rc) return rc;
-  VmBuf ba[3] = {vb(P, 96), vb(Q, 192), vb(cur().scratch[1].ptr, (long long)n)};
+  VmBuf ba[3] = {vb(P, 96), vb(Q, 192), vb(dbuf(MILLER_RAW), (long long)n)};
   rc = launch_named("miller_raw", n, ba, 3);
   if (rc) return rc;
   return raw_product_dev(out576, n);
+}
+
+// the final exponentiation of the Miller product: prod_i e(P_i, Q_i) -> out576
+int pairing_multi_dev(const void* P, const void* Q, void* out576, size_t n) {
+  int rc = ensure(MULTI_PRODUCT, 576);
+  if (!rc) rc = miller_product_dev(P, Q, dbuf(MULTI_PRODUCT), n);
+  if (rc) return rc;
+  VmBuf b[2] = {vb(dbuf(MULTI_PRODUCT), 576), vb(out576, 576)};
+  return launch_named("final_exp", 1, b, 2);
 }
 
 int sha_stage_dev(const void* hashes, void* out256, size_t n);
@@ -715,13 +602,12 @@ int sha_stage_dev(const void* hashes, void* out256, size_t n);
 // in the same program with H projective.  P: m x 96, mh: m x 32 (item 0 unused), Qgiven: m x 192
 // (used where given[i] != 0), given: m bytes.
 int aggregate_miller_dev(const void* P, const void* mh, const void* Qgiven, const void* given, void* out576, size_t m) {
-  NEED_READY();
-  int rc = ensure_scratch(1, (size_t)576 * m);
-  if (!rc) rc = ensure_scratch(3, (size_t)256 * m);
+  int rc = ensure(MILLER_RAW, (size_t)576 * m);
+  if (!rc) rc = ensure(SHA_OUT, (size_t)256 * m);
   if (rc) return rc;
-  rc = sha_stage_dev(mh, cur().scratch[3].ptr, m);
+  rc = sha_stage_dev(mh, dbuf(SHA_OUT), m);
   if (rc) return rc;
-  VmBuf bb[5] = {vb(P, 96), vb(cur().scratch[3].ptr, 256), vb(cur().scratch[1].ptr, (long long)m), vb(Qgiven, 192),
+  VmBuf bb[5] = {vb(P, 96), vb(dbuf(SHA_OUT), 256), vb(dbuf(MILLER_RAW), (long long)m), vb(Qgiven, 192),
                  vb(given, 1)};
   rc = launch_named("miller_hash_raw", m, bb, 5);
   if (rc) return rc;
@@ -740,7 +626,6 @@ int sha_stage_dev(const void* hashes, void* out256, size_t n) {
 
 // aggregation exponents T_i = H(i || pk_hash) mod n for i in [first, first + n) (util.py:46-49)
 int hash_pks_dev(const void* pk_hash32, uint32_t first, void* out, size_t n) {
-  NEED_READY();
   if (n == 0) return 0;
   int block = 256;
   long long grid = ((long long)n + block - 1) / block;
@@ -751,32 +636,29 @@ int hash_pks_dev(const void* pk_hash32, uint32_t first, void* out, size_t n) {
 }
 
 int hash_to_g2_dev(const void* hashes, void* out, size_t n) {
-  NEED_READY();
   if (n == 0) return 0;
-  int rc = ensure_scratch(3, (size_t)256 * n);
+  int rc = ensure(SHA_OUT, (size_t)256 * n);
   if (rc) return rc;
-  rc = sha_stage_dev(hashes, cur().scratch[3].ptr, n);
+  rc = sha_stage_dev(hashes, dbuf(SHA_OUT), n);
   if (rc) return rc;
-  VmBuf b[2] = {vb(cur().scratch[3].ptr, 256), vb(out, 192)};
+  VmBuf b[2] = {vb(dbuf(SHA_OUT), 256), vb(out, 192)};
   return launch_named("hash_to_g2", n, b, 2);
 }
 
 int verify_dev(const void* pk, const void* mh, const void* sig, void* ok, size_t n) {
-  NEED_READY();
   if (n == 0) return 0;
   // SHA stage, then ONE program that hashes to G2 and verifies: the hashed point enters the Miller
   // loop projective, its to_affine inversion is never computed
-  int rc = ensure_scratch(3, (size_t)256 * n);
+  int rc = ensure(SHA_OUT, (size_t)256 * n);
   if (rc) return rc;
-  rc = sha_stage_dev(mh, cur().scratch[3].ptr, n);
+  rc = sha_stage_dev(mh, dbuf(SHA_OUT), n);
   if (rc) return rc;
-  VmBuf b[4] = {vb(pk, 96), vb(cur().scratch[3].ptr, 256), vb(sig, 192), vb(ok, 1)};
+  VmBuf b[4] = {vb(pk, 96), vb(dbuf(SHA_OUT), 256), vb(sig, 192), vb(ok, 1)};
   return launch_named("verify_full", n, b, 4);
 }
 
 // one flag byte per affine point from a g?_subgroup-style program (programs/curve.py: build_subgroup_check)
 int point_flags_dev(const char* program, bool g2, const void* pts, void* ok, size_t n) {
-  NEED_READY();
   if (n == 0) return 0;
   VmBuf b[2] = {vb(pts, g2 ? 192 : 96), vb(ok, 1)};
   return launch_named(program, n, b, 2);
@@ -811,11 +693,11 @@ int and_flags_dev(void* ok, const FlagList& fl, size_t n) {
 }
 
 // strict verification: "pk in G1 and not infinity" (g1_keyvalidate, decided on the coordinates reduced mod q as the
-// pairing reads them) and "sig in G2" for the affine keys and signatures into scratch[13], appended to fl
+// pairing reads them) and "sig in G2" for the affine keys and signatures into buffer STRICT_FLAGS, appended to fl
 int strict_flags_dev(const void* pk, const void* sig, size_t n, FlagList& fl) {
-  int rc = ensure_scratch(13, 2 * n);
+  int rc = ensure(STRICT_FLAGS, 2 * n);
   if (rc) return rc;
-  uint8_t* f = (uint8_t*)cur().scratch[13].ptr;
+  uint8_t* f = (uint8_t*)dbuf(STRICT_FLAGS);
   rc = point_flags_dev("g1_keyvalidate", false, pk, f, n);
   if (!rc) rc = subgroup_check_dev(true, sig, f + n, n);
   fl.f[fl.n++] = f;
@@ -825,7 +707,6 @@ int strict_flags_dev(const void* pk, const void* sig, size_t n, FlagList& fl) {
 
 // strict: the verdict AND-ed with "pk in G1, pk not infinity, sig in G2" (b200bls.h)
 int verify_strict_dev(const void* pk, const void* mh, const void* sig, void* ok, size_t n) {
-  NEED_READY();
   if (n == 0) return 0;
   int rc = verify_dev(pk, mh, sig, ok, n);
   FlagList fl = {};
@@ -839,25 +720,24 @@ int verify_strict_dev(const void* pk, const void* mh, const void* sig, void* ok,
 // signature that does not decode (the reference raises ValueError) counts as a rejection.
 // strict: the subgroup checks of verify_strict_dev on the decoded points as well.
 int verify_wire_dev(const void* pk48, const void* mh, const void* sig96, void* ok, size_t n, bool strict = false) {
-  NEED_READY();
   if (n == 0) return 0;
-  int rc = ensure_scratch(6, (size_t)96 * n);
-  if (!rc) rc = ensure_scratch(11, (size_t)192 * n);
-  if (!rc) rc = ensure_scratch(7, n);
-  if (!rc) rc = ensure_scratch(8, n);
+  int rc = ensure(WIRE_PK, (size_t)96 * n);
+  if (!rc) rc = ensure(WIRE_SIG, (size_t)192 * n);
+  if (!rc) rc = ensure(WIRE_PK_OK, n);
+  if (!rc) rc = ensure(WIRE_SIG_OK, n);
   if (rc) return rc;
   StreamCtx& sc = cur();
-  VmBuf b1[3] = {vb(pk48, 48), vb(sc.scratch[6].ptr, 96), vb(sc.scratch[7].ptr, 1)};
+  VmBuf b1[3] = {vb(pk48, 48), vb(dbuf(WIRE_PK), 96), vb(dbuf(WIRE_PK_OK), 1)};
   rc = launch_named("g1_decompress", n, b1, 3);
   if (rc) return rc;
-  VmBuf b2[3] = {vb(sig96, 96), vb(sc.scratch[11].ptr, 192), vb(sc.scratch[8].ptr, 1)};
+  VmBuf b2[3] = {vb(sig96, 96), vb(dbuf(WIRE_SIG), 192), vb(dbuf(WIRE_SIG_OK), 1)};
   rc = launch_named("g2_decompress", n, b2, 3);
   if (rc) return rc;
-  rc = verify_dev(sc.scratch[6].ptr, mh, sc.scratch[11].ptr, ok, n);
+  rc = verify_dev(dbuf(WIRE_PK), mh, dbuf(WIRE_SIG), ok, n);
   if (rc) return rc;
-  FlagList fl = {{(const uint8_t*)sc.scratch[7].ptr, (const uint8_t*)sc.scratch[8].ptr}, 2};
+  FlagList fl = {{(const uint8_t*)dbuf(WIRE_PK_OK), (const uint8_t*)dbuf(WIRE_SIG_OK)}, 2};
   if (strict) {
-    rc = strict_flags_dev(sc.scratch[6].ptr, sc.scratch[11].ptr, n, fl);
+    rc = strict_flags_dev(dbuf(WIRE_PK), dbuf(WIRE_SIG), n, fl);
     if (rc) return rc;
   }
   return and_flags_dev(ok, fl, n);
@@ -877,45 +757,18 @@ __global__ void compress_pack_kernel(const uint8_t* __restrict__ aff, const uint
 }
 
 int compress_dev(bool g2, const void* aff, void* out, size_t n) {
-  NEED_READY();
   if (n == 0) return 0;
-  int rc = ensure_scratch(5, n);
+  int rc = ensure(CFLAGS, n);
   if (rc) return rc;
   int xb = g2 ? 96 : 48;
-  VmBuf b[2] = {vb(aff, 2 * xb), vb(cur().scratch[5].ptr, 1)};
+  VmBuf b[2] = {vb(aff, 2 * xb), vb(dbuf(CFLAGS), 1)};
   rc = launch_named(g2 ? "g2_cflag" : "g1_cflag", n, b, 2);
   if (rc) return rc;
   long long threads = (long long)n * (xb / 4);
   compress_pack_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, STREAM>>>(
-      (const uint8_t*)aff, (const uint8_t*)cur().scratch[5].ptr, (uint8_t*)out, (long long)n, xb);
+      (const uint8_t*)aff, (const uint8_t*)dbuf(CFLAGS), (uint8_t*)out, (long long)n, xb);
   CU(cudaGetLastError());
   g_ctx.launches++;
-  return 0;
-}
-
-// host-pointer wrapper around a device pipeline: ins/outs are (host ptr, bytes) pairs staged
-// through cur().staging[0..]
-struct HostIO {
-  const void* in;
-  void* out;
-  size_t bytes;
-};
-
-template <class F>
-int with_staging(const HostIO* io, int n_io, F&& body) {
-  NEED_READY();
-  void* dev[VM_MAX_BUFS];
-  for (int i = 0; i < n_io; i++) {
-    int rc = ensure_staging(i, io[i].bytes ? io[i].bytes : 1);
-    if (rc) return rc;
-    dev[i] = cur().staging[i].ptr;
-    if (io[i].in && io[i].bytes) CU(cudaMemcpyAsync(dev[i], io[i].in, io[i].bytes, cudaMemcpyHostToDevice, STREAM));
-  }
-  int rc = body(dev);
-  if (rc) return rc;
-  for (int i = 0; i < n_io; i++)
-    if (io[i].out && io[i].bytes) CU(cudaMemcpyAsync(io[i].out, dev[i], io[i].bytes, cudaMemcpyDeviceToHost, STREAM));
-  CU(cudaStreamSynchronize(STREAM));
   return 0;
 }
 
@@ -950,7 +803,7 @@ int b200bls_init(int device) {
   CU(cudaSetDevice(device));
   cudaDeviceProp prop;
   CU(cudaGetDeviceProperties(&prop, device));
-  c.sm_count = prop.multiProcessorCount;
+  c.policy.sm_count = prop.multiProcessorCount;
   for (auto& sc : c.sc) {
     CU(cudaStreamCreateWithFlags(&sc.stream, cudaStreamNonBlocking));
     CU(cudaEventCreateWithFlags(&sc.done, cudaEventDisableTiming));
@@ -983,6 +836,7 @@ int b200bls_init(int device) {
   for (uint32_t i = 0; i < n_prog; i++) {
     BlobEntry en;
     memcpy(&en, blob + 16 + i * sizeof(BlobEntry), sizeof(en));
+    if (en.shape < 1 || en.shape > N_SHAPES) return fail(B200BLS_E_PROGRAM, "bad program blob: shape %u", en.shape);
     DevProgram dp;
     dp.n_ins = (int)en.n_ins;
     dp.body_start = (int)en.body_start;
@@ -990,18 +844,7 @@ int b200bls_init(int device) {
     dp.n_slots = (int)en.n_slots;
     dp.n_cold = (int)en.n_cold;
     dp.n_tmem = (int)en.n_tmem;
-    dp.ctas = (int)en.ctas;
-    dp.ctas2 = dp.ctas;
-    if (dp.ctas == 4) {  // shape id 4 = the wide shape: 384 items per SM (one CTA of 384 threads, or two CTAs of 192 pairs)
-      dp.ctas = 1;
-      dp.threads = VM_NT_WIDE;
-      dp.ctas2 = 2;
-      dp.items = VM2_NT_WIDE / 2;
-    } else if (dp.ctas == 5) {  // shape id 5: one CTA of 512 threads (one-thread kernel only)
-      dp.ctas = 1;
-      dp.threads = VM_NT_XWIDE;
-      dp.ctas2 = 0;
-    }
+    dp.shape = (int)en.shape;
     {
       const unsigned char* code = blob + en.code_off;
       for (uint32_t k = 0; k < en.n_ins; k++) {
@@ -1023,11 +866,9 @@ int b200bls_init(int device) {
     c.programs[nm] = dp;
   }
   const char* kenv = getenv("B200BLS_KERNEL");
-  if (kenv && kenv[0] >= '0' && kenv[0] <= '2') c.kernel = kenv[0] - '0';
+  if (kenv && kenv[0] >= '0' && kenv[0] <= '2') c.policy.kernel = kenv[0] - '0';
   const char* env = getenv("B200BLS_CTAS_PER_SM");
-  if (env && env[0] >= '0' && env[0] <= '5') c.ctas_per_sm = env[0] - '0';
-  const char* ienv = getenv("B200BLS_ISOLATED_SHAPE");
-  c.isolated_shape = (ienv && ienv[0] >= '1' && ienv[0] <= '5') ? ienv[0] - '0' : 0;
+  if (env && env[0] >= '0' && env[0] <= '5') c.policy.ctas_per_sm = env[0] - '0';
   c.device = device;
   c.ready = true;
   return 0;
@@ -1044,15 +885,9 @@ void b200bls_shutdown(void) {
   }
   c.programs.clear();
   for (auto& sc : c.sc) {
-    for (auto& s : sc.scratch) {
+    for (auto& s : sc.bufs) {
       if (s.ptr) cudaFree(s.ptr);
-      s.ptr = nullptr;
-      s.cap = 0;
-    }
-    for (auto& s : sc.staging) {
-      if (s.ptr) cudaFree(s.ptr);
-      s.ptr = nullptr;
-      s.cap = 0;
+      s = Staging();
     }
     if (sc.cold) cudaFree(sc.cold);
     sc.cold = nullptr;
@@ -1069,17 +904,17 @@ void b200bls_shutdown(void) {
   c.device = -1;
 }
 
-int b200bls_sm_count(void) { return g_ctx.ready ? g_ctx.sm_count : 0; }
+int b200bls_sm_count(void) { return g_ctx.ready ? g_ctx.policy.sm_count : 0; }
 
 int b200bls_set_ctas_per_sm(int n) {
   std::lock_guard<std::mutex> lk(g_mu);
   if (n < 0 || n > 5)
     return fail(B200BLS_E_ARG, "ctas_per_sm must be 0 (auto), 1, 2, 3, 4 (one CTA of 384 threads) or 5 (one of 512)");
-  g_ctx.ctas_per_sm = n;
+  g_ctx.policy.ctas_per_sm = n;
   return 0;
 }
 
-int b200bls_get_ctas_per_sm(void) { return g_ctx.ctas_per_sm; }
+int b200bls_get_ctas_per_sm(void) { return g_ctx.policy.ctas_per_sm; }
 
 int b200bls_sync(void) {
   std::lock_guard<std::mutex> lk(g_mu);
@@ -1172,384 +1007,299 @@ int b200bls_timer_stop(float* ms) {
 uint64_t b200bls_launch_count(void) { return g_ctx.launches; }
 
 int b200bls_run_program_dev(const char* name, size_t n_items, void* const* bufs, const int64_t* strides, int n_bufs) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (n_bufs < 0 || n_bufs > VM_MAX_BUFS) return fail(B200BLS_E_ARG, "n_bufs out of range");
   DevBuf db[VM_MAX_BUFS];
   for (int i = 0; i < n_bufs; i++) {
     db[i].ptr = bufs[i];
     db[i].stride = (size_t)strides[i];
   }
-  return run_dev(name, n_items, db, n_bufs);
+  return locked([&] { return run_dev(name, n_items, db, n_bufs); });
 }
 
 int b200bls_program_info(const char* name, int* n_ins, int* n_slots, int* n_cold) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  if (!g_ctx.ready) return fail(B200BLS_E_NOT_INIT, "not initialised");
-  const DevProgram* pr = find_program(name);
-  if (!pr) return B200BLS_E_PROGRAM;
-  if (n_ins) *n_ins = pr->n_ins;
-  if (n_slots) *n_slots = pr->n_slots;
-  if (n_cold) *n_cold = pr->n_cold;
-  return 0;
+  return locked([&] {
+    const DevProgram* pr = find_program(name);
+    if (!pr) return B200BLS_E_PROGRAM;
+    if (n_ins) *n_ins = pr->n_ins;
+    if (n_slots) *n_slots = pr->n_slots;
+    if (n_cold) *n_cold = pr->n_cold;
+    return 0;
+  });
 }
 
 int b200bls_field_op_batch(int level, int op, const uint8_t* a, const uint8_t* b, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   char name[32];
   int rc = field_prog_name(level, op, name, sizeof(name));
   if (rc) return rc;
-  size_t w = 48 * (size_t)level;
-  HostBuf hb[3] = {{a, nullptr, w}, {op <= 2 ? b : nullptr, nullptr, w}, {nullptr, out, w}};
   if (!a || !out || (op <= 2 && !b)) return fail(B200BLS_E_ARG, "null buffer");
-  return run_host(name, n, hb, 3);
+  const size_t w = 48 * (size_t)level;
+  return run_host(name, n, {{a, nullptr, w}, {op <= 2 ? b : nullptr, nullptr, w}, {nullptr, out, w}});
 }
 
 int b200bls_field_op_batch_dev(int level, int op, const void* a, const void* b, void* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   char name[32];
   int rc = field_prog_name(level, op, name, sizeof(name));
   if (rc) return rc;
   size_t w = 48 * (size_t)level;
   DevBuf db[3] = {{a, w}, {b ? b : a, w}, {out, w}};
-  return run_dev(name, n, db, 3);
+  return locked([&] { return run_dev(name, n, db, 3); });
 }
 
 // ---- single-function parity entry points (programs/extras.py) ------------------------------------------
 int b200bls_field_frob_batch(int level, int i, const uint8_t* a, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!(level == 2 || level == 6 || level == 12) || i < 0 || i >= level)
     return fail(B200BLS_E_ARG, "field_frob: level %d, power %d (want level 2, 6 or 12 and 0 <= i < level)", level, i);
   if (!a || !out) return fail(B200BLS_E_ARG, "null buffer");
   char name[32];
   snprintf(name, sizeof(name), "f%d_frob%d", level, i);
   const size_t w = 48 * (size_t)level;
-  HostBuf hb[2] = {{a, nullptr, w}, {nullptr, out, w}};
-  return run_host(name, n, hb, 2);
+  return run_host(name, n, {{a, nullptr, w}, {nullptr, out, w}});
 }
 
 int b200bls_field_pow_batch(int level, const uint8_t* a, const uint8_t* e48, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!(level == 1 || level == 2 || level == 6 || level == 12)) return fail(B200BLS_E_ARG, "field_pow: bad level %d", level);
   if (!a || !e48 || !out) return fail(B200BLS_E_ARG, "null buffer");
   char name[32];
   snprintf(name, sizeof(name), "f%d_pow", level);
   const size_t w = 48 * (size_t)level;
-  HostBuf hb[3] = {{a, nullptr, w}, {e48, nullptr, 48}, {nullptr, out, w}};
-  return run_host(name, n, hb, 3);
+  return run_host(name, n, {{a, nullptr, w}, {e48, nullptr, 48}, {nullptr, out, w}});
 }
 
 int b200bls_field_sqrt_batch(int level, const uint8_t* a, uint8_t* out, uint8_t* ok, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!(level == 1 || level == 2)) return fail(B200BLS_E_ARG, "field_sqrt: level %d (want 1 or 2)", level);
   if (!a || !out || !ok) return fail(B200BLS_E_ARG, "null buffer");
   const size_t w = 48 * (size_t)level;
-  HostBuf hb[3] = {{a, nullptr, w}, {nullptr, out, w}, {nullptr, ok, 1}};
-  return run_host(level == 1 ? "f1_sqrt" : "f2_sqrt", n, hb, 3);
+  return run_host(level == 1 ? "f1_sqrt" : "f2_sqrt", n, {{a, nullptr, w}, {nullptr, out, w}, {nullptr, ok, 1}});
 }
 
 int b200bls_jacobian_op_batch(int g2, int op, const uint8_t* a, const uint8_t* b, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   static const char* kOps[4] = {"affine", "dbl", "add", "mul"};
   if (op < 0 || op > 3) return fail(B200BLS_E_ARG, "jacobian_op: op %d (0 to_affine, 1 double, 2 add, 3 scalar mult)", op);
   if (!a || !out || (op >= 2 && !b)) return fail(B200BLS_E_ARG, "null buffer");
   char name[32];
   snprintf(name, sizeof(name), "%s_j%s", g2 ? "g2" : "g1", kOps[op]);
   const size_t w = g2 ? 96 : 48;
-  HostBuf hb[3] = {{a, nullptr, 3 * w}, {op >= 2 ? b : nullptr, nullptr, op == 3 ? (size_t)32 : 3 * w}, {nullptr, out, 2 * w}};
-  return run_host(name, n, hb, 3);
+  return run_host(name, n, {{a, nullptr, 3 * w}, {op >= 2 ? b : nullptr, nullptr, op == 3 ? (size_t)32 : 3 * w},
+                            {nullptr, out, 2 * w}});
 }
 
 int b200bls_sw_encode_g2_batch(const uint8_t* t, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!t || !out) return fail(B200BLS_E_ARG, "null buffer");
-  HostBuf hb[2] = {{t, nullptr, 96}, {nullptr, out, 192}};
-  return run_host("sw_encode_g2", n, hb, 2);
+  return run_host("sw_encode_g2", n, {{t, nullptr, 96}, {nullptr, out, 192}});
 }
 
 int b200bls_g2_untwist_batch(const uint8_t* pts, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!pts || !out) return fail(B200BLS_E_ARG, "null buffer");
-  HostBuf hb[2] = {{pts, nullptr, 192}, {nullptr, out, 1152}};
-  return run_host("g2_untwist", n, hb, 2);
+  return run_host("g2_untwist", n, {{pts, nullptr, 192}, {nullptr, out, 1152}});
 }
 
 int b200bls_fq12_twist_batch(const uint8_t* pts, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!pts || !out) return fail(B200BLS_E_ARG, "null buffer");
-  HostBuf hb[2] = {{pts, nullptr, 1152}, {nullptr, out, 1152}};
-  return run_host("f12_twist", n, hb, 2);
+  return run_host("f12_twist", n, {{pts, nullptr, 1152}, {nullptr, out, 1152}});
 }
 
 int b200bls_g2_psi_batch(const uint8_t* pts, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!pts || !out) return fail(B200BLS_E_ARG, "null buffer");
-  HostBuf hb[2] = {{pts, nullptr, 192}, {nullptr, out, 192}};
-  return run_host("g2_psi", n, hb, 2);
+  return run_host("g2_psi", n, {{pts, nullptr, 192}, {nullptr, out, 192}});
 }
 
 int b200bls_pairing_batch(const uint8_t* P, const uint8_t* Q, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!P || !Q || !out) return fail(B200BLS_E_ARG, "null buffer");
-  HostBuf hb[3] = {{P, nullptr, 96}, {Q, nullptr, 192}, {nullptr, out, 576}};
-  return run_host("pairing", n, hb, 3);
+  return run_host("pairing", n, {{P, nullptr, 96}, {Q, nullptr, 192}, {nullptr, out, 576}});
 }
 
 int b200bls_pairing_batch_async(const uint8_t* P, const uint8_t* Q, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!P || !Q || !out) return fail(B200BLS_E_ARG, "null buffer");
-  HostBuf hb[3] = {{P, nullptr, 96}, {Q, nullptr, 192}, {nullptr, out, 576}};
-  return run_host("pairing", n, hb, 3, false);
+  return run_host("pairing", n, {{P, nullptr, 96}, {Q, nullptr, 192}, {nullptr, out, 576}}, true);
 }
 
 int b200bls_pairing_batch_dev(const void* P, const void* Q, void* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   DevBuf db[3] = {{P, 96}, {Q, 192}, {out, 576}};
-  return run_dev("pairing", n, db, 3);
+  return locked([&] { return run_dev("pairing", n, db, 3); });
 }
 
 int b200bls_final_exp_batch(const uint8_t* in, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!in || !out) return fail(B200BLS_E_ARG, "null buffer");
-  HostBuf hb[2] = {{in, nullptr, 576}, {nullptr, out, 576}};
-  return run_host("final_exp", n, hb, 2);
+  return run_host("final_exp", n, {{in, nullptr, 576}, {nullptr, out, 576}});
 }
 
 int b200bls_final_exp_batch_dev(const void* in, void* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   DevBuf db[2] = {{in, 576}, {out, 576}};
-  return run_dev("final_exp", n, db, 2);
+  return locked([&] { return run_dev("final_exp", n, db, 2); });
 }
 
 int b200bls_miller_loop_batch(const uint8_t* P, const uint8_t* Q, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!P || !Q || !out) return fail(B200BLS_E_ARG, "null buffer");
-  HostBuf hb[3] = {{P, nullptr, 96}, {Q, nullptr, 192}, {nullptr, out, 576}};
-  return run_host("miller_loop", n, hb, 3);
+  return run_host("miller_loop", n, {{P, nullptr, 96}, {Q, nullptr, 192}, {nullptr, out, 576}});
 }
 
 int b200bls_miller_loop_batch_dev(const void* P, const void* Q, void* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   DevBuf db[3] = {{P, 96}, {Q, 192}, {out, 576}};
-  return run_dev("miller_loop", n, db, 3);
+  return locked([&] { return run_dev("miller_loop", n, db, 3); });
 }
 
 
 // ---- curve ---------------------------------------------------------------------------------
 int b200bls_g1_scalar_mul_batch(const uint8_t* pts, const uint8_t* scalars, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!pts || !scalars || !out) return fail(B200BLS_E_ARG, "null buffer");
-  HostBuf hb[3] = {{pts, nullptr, 96}, {scalars, nullptr, 32}, {nullptr, out, 96}};
-  return run_host("g1_mul", n, hb, 3);
+  return run_host("g1_mul", n, {{pts, nullptr, 96}, {scalars, nullptr, 32}, {nullptr, out, 96}});
 }
 int b200bls_g1_scalar_mul_batch_dev(const void* pts, const void* scalars, void* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   DevBuf db[3] = {{pts, 96}, {scalars, 32}, {out, 96}};
-  return run_dev("g1_mul", n, db, 3);
+  return locked([&] { return run_dev("g1_mul", n, db, 3); });
 }
 int b200bls_g2_scalar_mul_batch(const uint8_t* pts, const uint8_t* scalars, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!pts || !scalars || !out) return fail(B200BLS_E_ARG, "null buffer");
-  HostBuf hb[3] = {{pts, nullptr, 192}, {scalars, nullptr, 32}, {nullptr, out, 192}};
-  return run_host("g2_mul", n, hb, 3);
+  return run_host("g2_mul", n, {{pts, nullptr, 192}, {scalars, nullptr, 32}, {nullptr, out, 192}});
 }
 int b200bls_g2_scalar_mul_batch_dev(const void* pts, const void* scalars, void* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   DevBuf db[3] = {{pts, 192}, {scalars, 32}, {out, 192}};
-  return run_dev("g2_mul", n, db, 3);
+  return locked([&] { return run_dev("g2_mul", n, db, 3); });
 }
 int b200bls_g1_add_batch(const uint8_t* a, const uint8_t* b, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!a || !b || !out) return fail(B200BLS_E_ARG, "null buffer");
-  HostBuf hb[3] = {{a, nullptr, 96}, {b, nullptr, 96}, {nullptr, out, 96}};
-  return run_host("g1_add", n, hb, 3);
+  return run_host("g1_add", n, {{a, nullptr, 96}, {b, nullptr, 96}, {nullptr, out, 96}});
 }
 int b200bls_g2_add_batch(const uint8_t* a, const uint8_t* b, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!a || !b || !out) return fail(B200BLS_E_ARG, "null buffer");
-  HostBuf hb[3] = {{a, nullptr, 192}, {b, nullptr, 192}, {nullptr, out, 192}};
-  return run_host("g2_add", n, hb, 3);
+  return run_host("g2_add", n, {{a, nullptr, 192}, {b, nullptr, 192}, {nullptr, out, 192}});
 }
 int b200bls_g1_sum_dev(const void* pts, void* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  return sum_dev(false, pts, out, n);
+  return locked([&] { return sum_dev(false, pts, out, n); });
 }
 int b200bls_g2_sum_dev(const void* pts, void* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  return sum_dev(true, pts, out, n);
+  return locked([&] { return sum_dev(true, pts, out, n); });
 }
 int b200bls_g1_sum(const uint8_t* pts, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!out || (n && !pts)) return fail(B200BLS_E_ARG, "null buffer");
   HostIO io[2] = {{pts, nullptr, 96 * n}, {nullptr, out, 96}};
   return with_staging(io, 2, [&](void** d) { return sum_dev(false, d[0], d[1], n); });
 }
 int b200bls_g2_sum(const uint8_t* pts, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!out || (n && !pts)) return fail(B200BLS_E_ARG, "null buffer");
   HostIO io[2] = {{pts, nullptr, 192 * n}, {nullptr, out, 192}};
   return with_staging(io, 2, [&](void** d) { return sum_dev(true, d[0], d[1], n); });
 }
 int b200bls_g1_decompress_batch(const uint8_t* in, uint8_t* out, uint8_t* ok, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!in || !out || !ok) return fail(B200BLS_E_ARG, "null buffer");
-  HostBuf hb[3] = {{in, nullptr, 48}, {nullptr, out, 96}, {nullptr, ok, 1}};
-  return run_host("g1_decompress", n, hb, 3);
+  return run_host("g1_decompress", n, {{in, nullptr, 48}, {nullptr, out, 96}, {nullptr, ok, 1}});
 }
 int b200bls_g2_decompress_batch(const uint8_t* in, uint8_t* out, uint8_t* ok, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!in || !out || !ok) return fail(B200BLS_E_ARG, "null buffer");
-  HostBuf hb[3] = {{in, nullptr, 96}, {nullptr, out, 192}, {nullptr, ok, 1}};
-  return run_host("g2_decompress", n, hb, 3);
+  return run_host("g2_decompress", n, {{in, nullptr, 96}, {nullptr, out, 192}, {nullptr, ok, 1}});
 }
 int b200bls_g1_compress_batch(const uint8_t* in, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!in || !out) return fail(B200BLS_E_ARG, "null buffer");
   HostIO io[2] = {{in, nullptr, 96 * n}, {nullptr, out, 48 * n}};
   return with_staging(io, 2, [&](void** d) { return compress_dev(false, d[0], d[1], n); });
 }
 int b200bls_g2_compress_batch(const uint8_t* in, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!in || !out) return fail(B200BLS_E_ARG, "null buffer");
   HostIO io[2] = {{in, nullptr, 192 * n}, {nullptr, out, 96 * n}};
   return with_staging(io, 2, [&](void** d) { return compress_dev(true, d[0], d[1], n); });
 }
 int b200bls_subgroup_check_batch(int g2, const uint8_t* pts, uint8_t* ok, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!pts || !ok) return fail(B200BLS_E_ARG, "null buffer");
   size_t w = g2 ? 192 : 96;
   HostIO io[2] = {{pts, nullptr, w * n}, {nullptr, ok, n}};
   return with_staging(io, 2, [&](void** d) { return subgroup_check_dev(g2 != 0, d[0], d[1], n); });
 }
 int b200bls_subgroup_check_batch_dev(int g2, const void* pts, void* ok, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  return subgroup_check_dev(g2 != 0, pts, ok, n);
+  return locked([&] { return subgroup_check_dev(g2 != 0, pts, ok, n); });
 }
 int b200bls_key_validate_batch(const uint8_t* pts, uint8_t* ok, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!pts || !ok) return fail(B200BLS_E_ARG, "null buffer");
   HostIO io[2] = {{pts, nullptr, 96 * n}, {nullptr, ok, n}};
   return with_staging(io, 2, [&](void** d) { return point_flags_dev("g1_keyvalidate", false, d[0], d[1], n); });
 }
 int b200bls_key_validate_batch_dev(const void* pts, void* ok, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  return point_flags_dev("g1_keyvalidate", false, pts, ok, n);
+  return locked([&] { return point_flags_dev("g1_keyvalidate", false, pts, ok, n); });
 }
 
 // ---- hashing, multi-pairing, verification ----------------------------------------------------
 int b200bls_hash_to_g2_batch(const uint8_t* hashes, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!hashes || !out) return fail(B200BLS_E_ARG, "null buffer");
   HostIO io[2] = {{hashes, nullptr, 32 * n}, {nullptr, out, 192 * n}};
   return with_staging(io, 2, [&](void** d) { return hash_to_g2_dev(d[0], d[1], n); });
 }
 int b200bls_hash_to_g2_batch_dev(const void* hashes, void* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  return hash_to_g2_dev(hashes, out, n);
+  return locked([&] { return hash_to_g2_dev(hashes, out, n); });
 }
 int b200bls_g1_msm(const uint8_t* pts, const uint8_t* scalars, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!out || (n && (!pts || !scalars))) return fail(B200BLS_E_ARG, "null buffer");
   HostIO io[3] = {{pts, nullptr, 96 * n}, {scalars, nullptr, 32 * n}, {nullptr, out, 96}};
   return with_staging(io, 3, [&](void** d) { return msm_dev(false, d[0], d[1], d[2], n); });
 }
 int b200bls_g1_msm_dev(const void* pts, const void* scalars, void* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  return msm_dev(false, pts, scalars, out, n);
+  return locked([&] { return msm_dev(false, pts, scalars, out, n); });
 }
 int b200bls_g2_msm(const uint8_t* pts, const uint8_t* scalars, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!out || (n && (!pts || !scalars))) return fail(B200BLS_E_ARG, "null buffer");
   HostIO io[3] = {{pts, nullptr, 192 * n}, {scalars, nullptr, 32 * n}, {nullptr, out, 192}};
   return with_staging(io, 3, [&](void** d) { return msm_dev(true, d[0], d[1], d[2], n); });
 }
 int b200bls_g2_msm_dev(const void* pts, const void* scalars, void* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  return msm_dev(true, pts, scalars, out, n);
+  return locked([&] { return msm_dev(true, pts, scalars, out, n); });
 }
 int b200bls_hash_pks(const uint8_t* pk_hash32, uint32_t first_index, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!pk_hash32 || !out) return fail(B200BLS_E_ARG, "null buffer");
   if ((unsigned long long)first_index + n > 0x100000000ull) return fail(B200BLS_E_ARG, "index does not fit 4 bytes");
   HostIO io[2] = {{pk_hash32, nullptr, 32}, {nullptr, out, 32 * n}};
   return with_staging(io, 2, [&](void** d) { return hash_pks_dev(d[0], first_index, d[1], n); });
 }
 int b200bls_hash_pks_dev(const void* pk_hash32, uint32_t first_index, void* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if ((unsigned long long)first_index + n > 0x100000000ull) return fail(B200BLS_E_ARG, "index does not fit 4 bytes");
-  return hash_pks_dev(pk_hash32, first_index, out, n);
+  return locked([&] { return hash_pks_dev(pk_hash32, first_index, out, n); });
 }
 int b200bls_miller_product(const uint8_t* P, const uint8_t* Q, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!out || (n && (!P || !Q))) return fail(B200BLS_E_ARG, "null buffer");
   HostIO io[3] = {{P, nullptr, 96 * n}, {Q, nullptr, 192 * n}, {nullptr, out, 576}};
   return with_staging(io, 3, [&](void** d) { return miller_product_dev(d[0], d[1], d[2], n); });
 }
 int b200bls_miller_product_dev(const void* P, const void* Q, void* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  return miller_product_dev(P, Q, out, n);
+  return locked([&] { return miller_product_dev(P, Q, out, n); });
 }
 int b200bls_pairing_multi(const uint8_t* P, const uint8_t* Q, uint8_t* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!out || (n && (!P || !Q))) return fail(B200BLS_E_ARG, "null buffer");
-  HostIO io[4] = {{P, nullptr, 96 * n}, {Q, nullptr, 192 * n}, {nullptr, nullptr, 576}, {nullptr, out, 576}};
-  return with_staging(io, 4, [&](void** d) {
-    int rc = miller_product_dev(d[0], d[1], d[2], n);
-    if (rc) return rc;
-    VmBuf b[2] = {vb(d[2], 576), vb(d[3], 576)};
-    return launch_named("final_exp", 1, b, 2);
-  });
+  HostIO io[3] = {{P, nullptr, 96 * n}, {Q, nullptr, 192 * n}, {nullptr, out, 576}};
+  return with_staging(io, 3, [&](void** d) { return pairing_multi_dev(d[0], d[1], d[2], n); });
 }
 int b200bls_pairing_multi_dev(const void* P, const void* Q, void* out, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  NEED_READY();
-  int rc = ensure_scratch(5, 576);
-  if (rc) return rc;
-  rc = miller_product_dev(P, Q, cur().scratch[5].ptr, n);
-  if (rc) return rc;
-  VmBuf b[2] = {vb(cur().scratch[5].ptr, 576), vb(out, 576)};
-  return launch_named("final_exp", 1, b, 2);
+  return locked([&] { return pairing_multi_dev(P, Q, out, n); });
 }
 int b200bls_verify_batch(const uint8_t* pk, const uint8_t* mh, const uint8_t* sig, uint8_t* ok, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!pk || !mh || !sig || !ok) return fail(B200BLS_E_ARG, "null buffer");
   HostIO io[4] = {{pk, nullptr, 96 * n}, {mh, nullptr, 32 * n}, {sig, nullptr, 192 * n}, {nullptr, ok, n}};
   return with_staging(io, 4, [&](void** d) { return verify_dev(d[0], d[1], d[2], d[3], n); });
 }
 int b200bls_verify_batch_dev(const void* pk, const void* mh, const void* sig, void* ok, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  return verify_dev(pk, mh, sig, ok, n);
+  return locked([&] { return verify_dev(pk, mh, sig, ok, n); });
 }
 
 int b200bls_verify_batch_wire(const uint8_t* pk48, const uint8_t* mh, const uint8_t* sig96, uint8_t* ok, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!pk48 || !mh || !sig96 || !ok) return fail(B200BLS_E_ARG, "null buffer");
   HostIO io[4] = {{pk48, nullptr, 48 * n}, {mh, nullptr, 32 * n}, {sig96, nullptr, 96 * n}, {nullptr, ok, n}};
   return with_staging(io, 4, [&](void** d) { return verify_wire_dev(d[0], d[1], d[2], d[3], n); });
 }
 int b200bls_verify_batch_wire_dev(const void* pk48, const void* mh, const void* sig96, void* ok, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  return verify_wire_dev(pk48, mh, sig96, ok, n);
+  return locked([&] { return verify_wire_dev(pk48, mh, sig96, ok, n); });
 }
 int b200bls_verify_batch_strict(const uint8_t* pk, const uint8_t* mh, const uint8_t* sig, uint8_t* ok, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!pk || !mh || !sig || !ok) return fail(B200BLS_E_ARG, "null buffer");
   HostIO io[4] = {{pk, nullptr, 96 * n}, {mh, nullptr, 32 * n}, {sig, nullptr, 192 * n}, {nullptr, ok, n}};
   return with_staging(io, 4, [&](void** d) { return verify_strict_dev(d[0], d[1], d[2], d[3], n); });
 }
 int b200bls_verify_batch_strict_dev(const void* pk, const void* mh, const void* sig, void* ok, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  return verify_strict_dev(pk, mh, sig, ok, n);
+  return locked([&] { return verify_strict_dev(pk, mh, sig, ok, n); });
 }
 int b200bls_verify_batch_wire_strict(const uint8_t* pk48, const uint8_t* mh, const uint8_t* sig96, uint8_t* ok,
                                      size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
   if (!pk48 || !mh || !sig96 || !ok) return fail(B200BLS_E_ARG, "null buffer");
   HostIO io[4] = {{pk48, nullptr, 48 * n}, {mh, nullptr, 32 * n}, {sig96, nullptr, 96 * n}, {nullptr, ok, n}};
   return with_staging(io, 4, [&](void** d) { return verify_wire_dev(d[0], d[1], d[2], d[3], n, true); });
 }
 int b200bls_verify_batch_wire_strict_dev(const void* pk48, const void* mh, const void* sig96, void* ok, size_t n) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  return verify_wire_dev(pk48, mh, sig96, ok, n, true);
+  return locked([&] { return verify_wire_dev(pk48, mh, sig96, ok, n, true); });
 }
 
 namespace {
@@ -1562,28 +1312,22 @@ const uint8_t kNegG1[96] = {
     0x4e, 0x6f, 0x38, 0xba, 0x0e, 0xcb, 0x75, 0x1b, 0xad, 0x54, 0xdc, 0xd6, 0xb9, 0x39, 0xc2, 0xca};
 
 // stages host inputs and leaves [e(-G1, sig) *] prod_i miller(pk_i, H(mh_i)) (big-endian, not
-// final-exponentiated) at staging[3]; sig may be null (a rank that does not own that pair)
+// final-exponentiated) in buffer AGG_MILLER; sig may be null (a rank that does not own that pair)
 int aggregate_miller_host(const uint8_t* sig, const uint8_t* pks, const uint8_t* mhs, size_t n) {
   const size_t lead = sig ? 1 : 0, m = n + lead;
   int rc;
-  if ((rc = ensure_staging(3, 576 * 2))) return rc;
-  if (m == 0) {
-    // an empty slice (a rank of a sharded verification that owns no pair) contributes the empty product:
-    // one, so that every rank still reaches the exchange
-    static const uint8_t kOne[48] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0,
-                                     0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 1};
-    CU(cudaMemsetAsync(cur().staging[3].ptr, 0, 576, STREAM));
-    CU(cudaMemcpyAsync(cur().staging[3].ptr, kOne, 48, cudaMemcpyHostToDevice, STREAM));
-    return 0;
-  }
-  if ((rc = ensure_staging(0, 96 * m))) return rc;
-  if ((rc = ensure_staging(1, 32 * m))) return rc;
-  if ((rc = ensure_staging(2, 192 * m))) return rc;
-  if ((rc = ensure_staging(4, m))) return rc;
-  uint8_t* dP = (uint8_t*)cur().staging[0].ptr;
-  uint8_t* dM = (uint8_t*)cur().staging[1].ptr;
-  uint8_t* dQ = (uint8_t*)cur().staging[2].ptr;
-  uint8_t* dG = (uint8_t*)cur().staging[4].ptr;
+  if ((rc = ensure(AGG_MILLER, 576 * 2))) return rc;
+  // an empty slice (a rank of a sharded verification that owns no pair) contributes the empty product: one, so that
+  // every rank still reaches the exchange
+  if (m == 0) return fq12_one_dev(dbuf(AGG_MILLER));
+  if ((rc = ensure(AGG_P, 96 * m))) return rc;
+  if ((rc = ensure(AGG_MH, 32 * m))) return rc;
+  if ((rc = ensure(AGG_Q, 192 * m))) return rc;
+  if ((rc = ensure(AGG_GIVEN, m))) return rc;
+  uint8_t* dP = (uint8_t*)dbuf(AGG_P);
+  uint8_t* dM = (uint8_t*)dbuf(AGG_MH);
+  uint8_t* dQ = (uint8_t*)dbuf(AGG_Q);
+  uint8_t* dG = (uint8_t*)dbuf(AGG_GIVEN);
   CU(cudaMemsetAsync(dQ, 0, 192 * m, STREAM));
   CU(cudaMemsetAsync(dG, 0, m, STREAM));
   if (sig) {
@@ -1596,31 +1340,30 @@ int aggregate_miller_host(const uint8_t* sig, const uint8_t* pks, const uint8_t*
     CU(cudaMemcpyAsync(dP + 96 * lead, pks, 96 * n, cudaMemcpyHostToDevice, STREAM));
     CU(cudaMemcpyAsync(dM + 32 * lead, mhs, 32 * n, cudaMemcpyHostToDevice, STREAM));
   }
-  return aggregate_miller_dev(dP, dM, dQ, dG, cur().staging[3].ptr, m);
+  return aggregate_miller_dev(dP, dM, dQ, dG, dbuf(AGG_MILLER), m);
 }
 }  // namespace
 
 // [e(-G1, sig) *] prod_i miller(pk_i, H(mh_i)), NOT final-exponentiated: one rank's partial of a
 // sharded aggregate verification (sig = NULL on the ranks that do not own the signature pair)
 int b200bls_aggregate_miller(const uint8_t* sig, const uint8_t* pks, const uint8_t* mhs, size_t n, uint8_t* out576) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  NEED_READY();
-  if (!out576 || (n && (!pks || !mhs))) return fail(B200BLS_E_ARG, "null buffer");
-  int rc = aggregate_miller_host(sig, pks, mhs, n);
-  if (rc) return rc;
-  CU(cudaMemcpyAsync(out576, cur().staging[3].ptr, 576, cudaMemcpyDeviceToHost, STREAM));
-  CU(cudaStreamSynchronize(STREAM));
-  return 0;
+  return locked([&] {
+    if (!out576 || (n && (!pks || !mhs))) return fail(B200BLS_E_ARG, "null buffer");
+    int rc = aggregate_miller_host(sig, pks, mhs, n);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(out576, dbuf(AGG_MILLER), 576, cudaMemcpyDeviceToHost, STREAM));
+    CU(cudaStreamSynchronize(STREAM));
+    return 0;
+  });
 }
 
 namespace {
 // enqueues the whole aggregate verification on the selected stream, result byte -> *ok (host)
 int aggregate_verify_enqueue(const uint8_t* sig, const uint8_t* pks, const uint8_t* mhs, size_t n, uint8_t* ok) {
-  NEED_READY();
   if (!sig || !ok || (n && (!pks || !mhs))) return fail(B200BLS_E_ARG, "null buffer");
   int rc = aggregate_miller_host(sig, pks, mhs, n);
   if (rc) return rc;
-  uint8_t* dF = (uint8_t*)cur().staging[3].ptr;
+  uint8_t* dF = (uint8_t*)dbuf(AGG_MILLER);
   VmBuf b[2] = {vb(dF, 576), vb(dF + 576, 1)};
   if ((rc = launch_named("final_exp_check", 1, b, 2))) return rc;
   CU(cudaMemcpyAsync(ok, dF + 576, 1, cudaMemcpyDeviceToHost, STREAM));
@@ -1631,11 +1374,12 @@ int aggregate_verify_enqueue(const uint8_t* sig, const uint8_t* pks, const uint8
 // e(-G1, sig) * prod_i e(pk_i, H(mh_i)) == 1 for distinct message hashes and unit exponents:
 // the core of BLS.verify (bls_py/bls.py:194-201) after its host-side grouping
 int b200bls_aggregate_verify(const uint8_t* sig, const uint8_t* pks, const uint8_t* mhs, size_t n, uint8_t* ok) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  int rc = aggregate_verify_enqueue(sig, pks, mhs, n, ok);
-  if (rc) return rc;
-  CU(cudaStreamSynchronize(STREAM));
-  return 0;
+  return locked([&] {
+    int rc = aggregate_verify_enqueue(sig, pks, mhs, n, ok);
+    if (rc) return rc;
+    CU(cudaStreamSynchronize(STREAM));
+    return 0;
+  });
 }
 
 // the same without waiting: several aggregate verifications (on different library streams,
@@ -1643,8 +1387,7 @@ int b200bls_aggregate_verify(const uint8_t* sig, const uint8_t* pks, const uint8
 // b200bls_sync(); the input buffers must stay untouched until then (pinned memory lets the copies
 // overlap other streams' kernels).
 int b200bls_aggregate_verify_async(const uint8_t* sig, const uint8_t* pks, const uint8_t* mhs, size_t n, uint8_t* ok) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  return aggregate_verify_enqueue(sig, pks, mhs, n, ok);
+  return locked([&] { return aggregate_verify_enqueue(sig, pks, mhs, n, ok); });
 }
 
 // ---- multi-GPU: one process per GPU, one tiny all-gather per sharded reduction (comm.cuh) -------------------
@@ -1757,7 +1500,7 @@ int gather_partials(const void* src_dev, size_t bytes, int use_nccl, void** gath
     *gathered_dev = c.gather_dev;
     return 0;
   }
-  int rc = ensure_staging(5, (size_t)c.world * bytes);
+  int rc = ensure(GATHERED, (size_t)c.world * bytes);
   if (rc) return rc;
   static thread_local unsigned char mine[COMM_SLOT_BYTES];
   static thread_local unsigned char all[COMM_MAX_RANKS * 1024];
@@ -1765,8 +1508,8 @@ int gather_partials(const void* src_dev, size_t bytes, int use_nccl, void** gath
   CU(cudaMemcpyAsync(mine, src_dev, bytes, cudaMemcpyDeviceToHost, STREAM));
   CU(cudaStreamSynchronize(STREAM));
   if (comm_allgather_host(c, mine, all, bytes) != 0) return fail(B200BLS_E_CUDA, "host gather timed out");
-  CU(cudaMemcpyAsync(cur().staging[5].ptr, all, (size_t)c.world * bytes, cudaMemcpyHostToDevice, STREAM));
-  *gathered_dev = cur().staging[5].ptr;
+  CU(cudaMemcpyAsync(dbuf(GATHERED), all, (size_t)c.world * bytes, cudaMemcpyHostToDevice, STREAM));
+  *gathered_dev = dbuf(GATHERED);
   return 0;
 }
 }  // namespace
@@ -1778,50 +1521,50 @@ int gather_partials(const void* src_dev, size_t bytes, int use_nccl, void** gath
 // every rank returns the same *ok (bls_py/bls.py:194-201 over a sharded message list).
 int b200bls_aggregate_verify_sharded(const uint8_t* sig, const uint8_t* pks, const uint8_t* mhs, size_t n, int use_nccl,
                                      uint8_t* ok) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  NEED_READY();
-  if (!ok || (n && (!pks || !mhs))) return fail(B200BLS_E_ARG, "null buffer");
-  if (g_comm.rank == 0 && !sig) return fail(B200BLS_E_ARG, "rank 0 needs the signature");
-  int rc = aggregate_miller_host(g_comm.rank == 0 ? sig : nullptr, pks, mhs, n);
-  if (rc) return rc;
-  void* parts = nullptr;
-  if ((rc = gather_partials(cur().staging[3].ptr, 576, use_nccl, &parts))) return rc;
-  // product of the per-rank values: world - 1 Fq12 products on the device, then the final exponentiation check
-  if ((rc = ensure_staging(6, 576 + 16))) return rc;
-  uint8_t* acc = (uint8_t*)cur().staging[6].ptr;
-  CU(cudaMemcpyAsync(acc, parts, 576, cudaMemcpyDeviceToDevice, STREAM));
-  for (int r = 1; r < g_comm.world; r++) {
-    DevBuf db[3] = {{acc, 576}, {(uint8_t*)parts + 576 * (size_t)r, 576}, {acc, 576}};
-    if ((rc = run_dev("f12_mul", 1, db, 3))) return rc;
-  }
-  VmBuf b[2] = {vb(acc, 576), vb(acc + 576, 1)};
-  if ((rc = launch_named("final_exp_check", 1, b, 2))) return rc;
-  CU(cudaMemcpyAsync(ok, acc + 576, 1, cudaMemcpyDeviceToHost, STREAM));
-  CU(cudaStreamSynchronize(STREAM));
-  return 0;
+  return locked([&] {
+    if (!ok || (n && (!pks || !mhs))) return fail(B200BLS_E_ARG, "null buffer");
+    if (g_comm.rank == 0 && !sig) return fail(B200BLS_E_ARG, "rank 0 needs the signature");
+    int rc = aggregate_miller_host(g_comm.rank == 0 ? sig : nullptr, pks, mhs, n);
+    if (rc) return rc;
+    void* parts = nullptr;
+    if ((rc = gather_partials(dbuf(AGG_MILLER), 576, use_nccl, &parts))) return rc;
+    // product of the per-rank values: world - 1 Fq12 products on the device, then the final exponentiation check
+    if ((rc = ensure(SHARD_ACC, 576 + 16))) return rc;
+    uint8_t* acc = (uint8_t*)dbuf(SHARD_ACC);
+    CU(cudaMemcpyAsync(acc, parts, 576, cudaMemcpyDeviceToDevice, STREAM));
+    for (int r = 1; r < g_comm.world; r++) {
+      DevBuf db[3] = {{acc, 576}, {(uint8_t*)parts + 576 * (size_t)r, 576}, {acc, 576}};
+      if ((rc = run_dev("f12_mul", 1, db, 3))) return rc;
+    }
+    VmBuf b[2] = {vb(acc, 576), vb(acc + 576, 1)};
+    if ((rc = launch_named("final_exp_check", 1, b, 2))) return rc;
+    CU(cudaMemcpyAsync(ok, acc + 576, 1, cudaMemcpyDeviceToHost, STREAM));
+    CU(cudaStreamSynchronize(STREAM));
+    return 0;
+  });
 }
 
 // Sum of points sharded over the ranks (BLS.aggregate_sigs_simple / aggregate_pub_keys(secure=False),
 // bls.py:13-26, 204-223): pts_dev is THIS rank's device-resident slice of n affine points; every rank reduces
 // its slice to one affine point, the points are all-gathered and summed on every rank.  out: 96 / 192 host bytes.
 int b200bls_point_sum_sharded_dev(int g2, const void* pts_dev, size_t n, int use_nccl, uint8_t* out) {
-  std::lock_guard<std::mutex> lk(g_mu);
-  NEED_READY();
-  if (!out) return fail(B200BLS_E_ARG, "null buffer");
-  const size_t w = g2 ? 192 : 96;
-  int rc = ensure_staging(6, 2 * w);
-  if (rc) return rc;
-  uint8_t* part = (uint8_t*)cur().staging[6].ptr;
-  if ((rc = sum_dev(g2 != 0, pts_dev, part, n))) return rc;
-  void* parts = nullptr;
-  if ((rc = gather_partials(part, w, use_nccl, &parts))) return rc;
-  if (g_comm.world > 1) {
-    if ((rc = sum_dev(g2 != 0, parts, part + w, (size_t)g_comm.world))) return rc;
-    part += w;
-  }
-  CU(cudaMemcpyAsync(out, part, w, cudaMemcpyDeviceToHost, STREAM));
-  CU(cudaStreamSynchronize(STREAM));
-  return 0;
+  return locked([&] {
+    if (!out) return fail(B200BLS_E_ARG, "null buffer");
+    const size_t w = g2 ? 192 : 96;
+    int rc = ensure(SHARD_ACC, 2 * w);
+    if (rc) return rc;
+    uint8_t* part = (uint8_t*)dbuf(SHARD_ACC);
+    if ((rc = sum_dev(g2 != 0, pts_dev, part, n))) return rc;
+    void* parts = nullptr;
+    if ((rc = gather_partials(part, w, use_nccl, &parts))) return rc;
+    if (g_comm.world > 1) {
+      if ((rc = sum_dev(g2 != 0, parts, part + w, (size_t)g_comm.world))) return rc;
+      part += w;
+    }
+    CU(cudaMemcpyAsync(out, part, w, cudaMemcpyDeviceToHost, STREAM));
+    CU(cudaStreamSynchronize(STREAM));
+    return 0;
+  });
 }
 
 }  // extern "C"
