@@ -228,6 +228,23 @@ int b200bls_sw_encode_g2_batch(const uint8_t* t, uint8_t* out, size_t n);
 /* hash_to_point_prehashed_Fq2 (ec.py:528-550): n x 32-byte message hashes -> n x 192 bytes. */
 int b200bls_hash_to_g2_batch(const uint8_t* hashes, uint8_t* out, size_t n);
 int b200bls_hash_to_g2_batch_dev(const void* hashes, void* out, size_t n);
+/* PrivateKey.sign_prehashed (keys.py:128-132) for n (secret key, message hash) pairs: sig_i = sk_i * H(mh_i).
+ * sk32: n x 32-byte big-endian secret keys (any value below 2^256; the signature is that of sk mod n), mh32: n x 32
+ * bytes.  wire = 0: sig = n x 192 affine bytes; wire = 1: sig = n x 96 Signature.serialize() bytes.  The bytes are
+ * those of the reference.  One device pass per batch: the SHA stage, a split of sk mod n into four base-|x| digits,
+ * and one program that hashes to G2 and runs a 64-step ladder over the digits and the endomorphism psi (0.63x the
+ * Montgomery products of b200bls_hash_to_g2_batch followed by b200bls_g2_scalar_mul_batch).  n = 0 does nothing.
+ * Secret keys: the library's device copies -- the staged copy of sk32 in the host-buffer form and the digit buffer
+ * in both forms -- are zeroed on the stream after their last reader, before the call returns.  The caller of the
+ * _dev form owns its sk32 buffer and clears it.  Not constant-time: the inversion and the regions that warps skip
+ * depend on the data, as in the scalar multiplications above. */
+int b200bls_sign_batch(int wire, const uint8_t* sk32, const uint8_t* mh32, uint8_t* sig, size_t n);
+int b200bls_sign_batch_dev(int wire, const void* sk32, const void* mh32, void* sig, size_t n);
+/* PrivateKey.get_public_key (keys.py:119-121): pk_i = sk_i * G1, from the same digits with a table of multiples of
+ * G1 fixed at build time (0.38x the products of b200bls_g1_scalar_mul_batch).  wire = 0: pk = n x 96 affine bytes;
+ * wire = 1: n x 48 PublicKey.serialize() bytes.  Secret-key handling and timing as for b200bls_sign_batch. */
+int b200bls_public_key_batch(int wire, const uint8_t* sk32, uint8_t* pk, size_t n);
+int b200bls_public_key_batch_dev(int wire, const void* sk32, void* pk, size_t n);
 /* hash_pks (util.py:36-50), the per-key part: out[i] = SHA256(uint32_be(first_index + i) ||
  * pk_hash) mod n as 32 big-endian bytes (the scalar format of the scalar-multiplication entry
  * points), pk_hash = SHA256(pk_1 || ... || pk_N) computed by the caller.  These are the

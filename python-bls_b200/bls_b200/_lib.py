@@ -98,6 +98,10 @@ def _load():
         "b200bls_hash_pks_dev": (i32, [vp, ctypes.c_uint32, vp, sz]),
         "b200bls_hash_to_g2_batch": (i32, [vp, vp, sz]),
         "b200bls_hash_to_g2_batch_dev": (i32, [vp, vp, sz]),
+        "b200bls_sign_batch": (i32, [i32, vp, vp, vp, sz]),
+        "b200bls_sign_batch_dev": (i32, [i32, vp, vp, vp, sz]),
+        "b200bls_public_key_batch": (i32, [i32, vp, vp, sz]),
+        "b200bls_public_key_batch_dev": (i32, [i32, vp, vp, sz]),
         "b200bls_verify_batch": (i32, [vp, vp, vp, vp, sz]),
         "b200bls_verify_batch_dev": (i32, [vp, vp, vp, vp, sz]),
         "b200bls_aggregate_verify": (i32, [vp, vp, vp, sz, vp]),

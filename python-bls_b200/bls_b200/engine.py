@@ -10,6 +10,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import as_u8, check, lib, ptr
+from .util import GROUP_ORDER
 
 FIELD_OPS = {"add": 0, "sub": 1, "mul": 2, "sqr": 3, "neg": 4, "inv": 5}
 
@@ -302,6 +303,40 @@ def hash_to_g2(hashes):
         raise ValueError("bad buffer size")
     out = np.empty(n * 192, dtype=np.uint8)
     check(lib.b200bls_hash_to_g2_batch(ptr(hashes), ptr(out), n))
+    return out
+
+
+def _secret_keys(sks):
+    """ints (taken mod the group order) or n x 32 big-endian bytes -> uint8 array of n x 32 bytes"""
+    if isinstance(sks, (bytes, bytearray, np.ndarray)):
+        sks = as_u8(sks)
+        if sks.size % 32:
+            raise ValueError("secret keys are 32 bytes each")
+        return sks
+    return np.frombuffer(b"".join((int(k) % GROUP_ORDER).to_bytes(32, "big") for k in sks), dtype=np.uint8)
+
+
+def sign_batch(sks, hashes, wire=False):
+    """PrivateKey.sign_prehashed for n (secret key, 32-byte message hash) pairs in one device pass: sks are ints or
+    n x 32 big-endian bytes -> n x 192 affine bytes, or n x 96 Signature.serialize() bytes with wire=True"""
+    _lib.init()
+    sks, hashes = _secret_keys(sks), as_u8(hashes)
+    n = hashes.size // 32
+    if hashes.size != 32 * n or sks.size != 32 * n:
+        raise ValueError("bad buffer sizes")
+    out = np.empty(n * (96 if wire else 192), dtype=np.uint8)
+    check(lib.b200bls_sign_batch(int(bool(wire)), ptr(sks), ptr(hashes), ptr(out), n))
+    return out
+
+
+def public_keys(sks, wire=False):
+    """PrivateKey.get_public_key for n secret keys (ints or n x 32 big-endian bytes) in one device pass -> n x 96
+    affine bytes, or n x 48 PublicKey.serialize() bytes with wire=True"""
+    _lib.init()
+    sks = _secret_keys(sks)
+    n = sks.size // 32
+    out = np.empty(n * (48 if wire else 96), dtype=np.uint8)
+    check(lib.b200bls_public_key_batch(int(bool(wire)), ptr(sks), ptr(out), n))
     return out
 
 

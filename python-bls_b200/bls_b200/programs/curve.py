@@ -226,6 +226,35 @@ class Curve:
             acc = tuple(self.sel(nz, a, b) for a, b in zip(s, acc))
         return acc
 
+    def digit_ladder(self, table, digit_buf):
+        """sum_i d_i B_i for the four 64-bit digits d_i of the item's record in `digit_buf` (csrc/scalar_split.h: digit
+        i in bits [64 i, 64 i + 64)), as ONE joint ladder of 64 steps, MSB first.  table[m] = (x, y) is the affine sum of
+        the B_i over the set bits i of m (table[0] is never used but must be some value); an entry may be a constant
+        (int for G1, pair for G2), loaded again in every step instead of being kept live.  A step is one doubling, a
+        4-flag selection of the entry and one complete mixed addition; when all four bits are clear the accumulator is
+        kept.  The entries must not be infinity (B_i of order n: a sum of distinct (-a)^i is a non-zero integer of
+        magnitude below n).  The additions stay complete: the accumulator equals +-(entry) exactly when a relation
+        sum c_i (-a)^i = 0 mod n with |c_i| < a holds, and nothing rules that out."""
+        prog = self.prog
+        get = (lambda v: self.const(v) if isinstance(v, (int, tuple)) else v)
+        no_inf = prog.flag_const(0)
+        acc = None
+        for j in range(63, -1, -1):
+            f = [prog.flag_bit(digit_buf, 64 * i + j) for i in range(4)]
+            level = table
+            for fi in f:
+                level = [(self.sel(fi, get(b[0]), get(a[0])), self.sel(fi, get(b[1]), get(a[1])))
+                         for a, b in zip(level[0::2], level[1::2])]
+            tx, ty = level[0]
+            nz = (f[0] | f[1]) | (f[2] | f[3])
+            if acc is None:
+                acc = (tx, ty, self.sel(nz, self.const(1), self.const(0)))
+                continue
+            acc = self.double(acc)
+            s = self.add(acc, (tx, ty), mixed=True, inf2=no_inf)
+            acc = tuple(self.sel(nz, a, b) for a, b in zip(s, acc))
+        return acc
+
     def subgroup_ladder(self, x, y, inf):
         """the Jacobian multiple in_subgroup compares with the endomorphism image: [|x|] P on G2, [x^2] P =
         [|x|]([|x|] P) on G1.  Complete additions: on a point of small order the accumulator can equal P at an
@@ -647,6 +676,60 @@ def build_subgroup_check(g2, key=False):
         prog.store_flag(1, 0, f & ~inf if key else f)
         return prog
     return build
+
+
+def _g1_aff_add(p, q):
+    """affine sum of two distinct, non-opposite points of E(Fq) (build-time constants only)"""
+    lam = (q[1] - p[1]) * pow(q[0] - p[0], -1, Q) % Q
+    x = (lam * lam - p[0] - q[0]) % Q
+    return (x, (lam * (p[0] - x) - p[1]) % Q)
+
+
+def _g1_aff_mul(k, p):
+    """k P for 0 < k < n by double-and-add on affine points (build-time constants only)"""
+    acc = None
+    for bit in bin(k)[2:]:
+        if acc is not None:
+            lam = 3 * acc[0] * acc[0] * pow(2 * acc[1], -1, Q) % Q
+            x = (lam * lam - 2 * acc[0]) % Q
+            acc = (x, (lam * (acc[0] - x) - acc[1]) % Q)
+        if bit == "1":
+            acc = p if acc is None else _g1_aff_add(acc, p)
+    return acc
+
+
+def _g1_pubkey_table():
+    """entry m = sum of [a^i] G1 over the set bits i of m (a = |x|); entry 0 repeats G1 (never selected)"""
+    from .hashg2 import X_ABS
+    base = [G1_GEN]
+    for _ in range(3):
+        base.append(_g1_aff_mul(X_ABS, base[-1]))
+    table = [G1_GEN]
+    for m in range(1, 16):
+        pt = None
+        for i in range(4):
+            if m >> i & 1:
+                pt = base[i] if pt is None else _g1_aff_add(pt, base[i])
+        table.append(pt)
+    return table
+
+
+G1_PUBKEY_TABLE = _g1_pubkey_table()
+
+
+def build_pubkey():
+    """PrivateKey.get_public_key (keys.py:119-121): sk * G1 from the digit record of sk mod n (csrc/scalar_split.h).
+    buffers: 0 = digit records (32 B), 1 = out (affine G1, 96 B), 2 = compression flag byte (1 iff y > q//2, the
+    flag g1_cflag computes).  The base point is fixed, so the table of the joint ladder ([a^i] G1 and their subset
+    sums, G1_PUBKEY_TABLE) is constants: 64 doublings and 64 mixed additions, against 255 doublings and 128 additions
+    of g1_mul."""
+    prog = Program("g1_pubkey")
+    prog.begin_body()
+    c = Curve(prog, False)
+    x, y = c.to_affine(c.digit_ladder(G1_PUBKEY_TABLE, 0))
+    c.store_affine(1, 0, (x, y))
+    prog.store_flag(2, 0, y.gt_half())
+    return prog
 
 
 def build_compress_flag(g2):

@@ -199,6 +199,69 @@ def hash_to_g2(prog, buf, affine=True):
     return c.to_affine(r) if affine else r
 
 
+# -psi^3(x, y) = (conj(x) PSI3_CX, conj(y) PSI_CY): psi^2 scales x by the Fq constant PSI2_CX and negates y
+PSI3_CX = (PSI2_CX * PSI_CX[0] % Q, PSI2_CX * PSI_CX[1] % Q)
+
+
+def sign_table(c, x, y):
+    """the 16-entry table of Curve.digit_ladder for an affine point P = (x, y) of G2 (not infinity):
+    B = (P, -psi P, psi^2 P, -psi^3 P) = ([1] P, [a] P, [a^2] P, [a^3] P), since psi acts on G2 as [x] = [-a];
+    entry m = sum of B_i over the set bits of m.  11 mixed additions, then ONE inversion for their 11 Z coordinates."""
+    prog = c.prog
+    cx, cy = prog.const2(PSI_CX), prog.const2(PSI_CY)
+    xc, yc = x.conj(), y.conj()
+    b = [(x, y), (xc * cx, -(yc * cy)), (x * prog.const1(PSI2_CX), -y), (xc * prog.const2(PSI3_CX), yc * cy)]
+    one, no_inf = c.const(1), prog.flag_const(0)
+    jac = {}
+    for hi in range(1, 4):                       # two base points: 3, 5, 6, 9, 10, 12
+        for lo in range(hi):
+            jac[(1 << hi) | (1 << lo)] = c.add((b[hi][0], b[hi][1], one), b[lo], mixed=True, inf2=no_inf)
+    for m, lo, hi in ((7, 3, 2), (11, 3, 3), (13, 5, 3), (14, 6, 3), (15, 7, 3)):
+        jac[m] = c.add(jac[lo], b[hi], mixed=True, inf2=no_inf)
+    # Montgomery's simultaneous inversion of the Z coordinates (none is zero: the entries are not infinity)
+    ms = sorted(jac)
+    pre = [jac[ms[0]][2]]
+    for m in ms[1:]:
+        pre.append(pre[-1] * jac[m][2])
+    inv = c.inv(pre[-1])
+    table = [None] * 16
+    for k in range(len(ms) - 1, -1, -1):
+        X, Y, Z = jac[ms[k]]
+        zi = inv * pre[k - 1] if k else inv
+        if k:
+            inv = inv * Z
+        zi2 = zi.sqr()
+        table[ms[k]] = (X * zi2, Y * (zi2 * zi))
+    for i in range(4):
+        table[1 << i] = b[i]
+    table[0] = b[0]
+    return table
+
+
+def build_sign():
+    """PrivateKey.sign_prehashed (keys.py:128-132): sk * H(h) for one message hash, from the SHA stage output and the
+    digit record of sk mod n (csrc/scalar_split.h).  buffers: 0 = SHA stage output (256 B), 1 = digit records (32 B),
+    2 = out (affine G2, 192 B), 3 = compression flag byte (1 iff y.c1 > q//2, the flag g2_cflag computes).
+    The hashed point is in G2, where psi = [-a]: k = d0 + d1 a + d2 a^2 + d3 a^3 gives
+    k H = d0 H + d1 (-psi H) + d2 psi^2 H + d3 (-psi^3 H), one 64-step joint ladder (Curve.digit_ladder) instead of
+    the 128-step two-bit ladder of g2_mul.  A hashed point at infinity gives the zero signature."""
+    prog = Program("g2_sign")
+    prog.begin_body()
+    c = Curve(prog, True)
+    r = hash_to_g2(prog, 0, affine=False)
+    inf = r[2].is_zero()
+    x, y = c.to_affine(r)
+    # infinity has no table without zero Z coordinates: ladder on the generator instead and discard the result
+    x = prog.sel2(inf, prog.const2(G2_GEN[0]), x)
+    y = prog.sel2(inf, prog.const2(G2_GEN[1]), y)
+    sx, sy = c.to_affine(c.digit_ladder(sign_table(c, x, y), 1))
+    zero = prog.const2((0, 0))
+    sx, sy = prog.sel2(inf, zero, sx), prog.sel2(inf, zero, sy)
+    c.store_affine(2, 0, (sx, sy))
+    prog.store_flag(3, 0, sy.c1.gt_half())
+    return prog
+
+
 def build_hash_to_g2():
     """buffers: 0 = SHA stage output (256 B per item), 1 = out (affine G2, 192 B)"""
     prog = Program("hash_to_g2")

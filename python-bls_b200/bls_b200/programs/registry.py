@@ -69,6 +69,8 @@ for _g2 in (False, True):
     PROGRAMS[_p + "_cflag"] = curve.build_compress_flag(_g2)
     PROGRAMS[_p + "_subgroup"] = curve.build_subgroup_check(_g2)
 PROGRAMS["g1_keyvalidate"] = curve.build_subgroup_check(False, key=True)
+PROGRAMS["g2_sign"] = hashg2.build_sign
+PROGRAMS["g1_pubkey"] = curve.build_pubkey
 
 
 # programs assembled for the one-CTA-per-SM shape only (seam / parity utilities, never launched in bulk)

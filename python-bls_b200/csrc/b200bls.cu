@@ -21,6 +21,7 @@
 #include "comm.cuh"
 #include "sha256.cuh"
 #include "gen/vm_isa.h"
+#include "scalar_split.h"
 #include "vm_launch.h"
 #include "vm_plan.h"
 
@@ -98,7 +99,12 @@ enum Buf {
   STRICT_FLAGS,             // strict_flags_dev: key and signature subgroup flags
   CFLAGS,                   // compress_dev: the flag bit of every point
   MULTI_PRODUCT = CFLAGS,   // b200bls_pairing_multi_dev (calls miller_product_dev): the Miller product
-  N_BUFS
+  // sign_dev and public_key_dev call neither msm_dev nor verify_wire_dev, and neither runs inside them; they take the
+  // three MSM buffers that verify_wire_dev leaves alone
+  SIGN_DIGITS = MSM_MONT,   // the base-a digits of sk mod n (scalar_split.h): secret, zeroed after the program
+  SIGN_AFFINE = MSM_IDX,    // wire output: the affine points before the compression pack
+  SIGN_FLAGS = MSM_SEGMENTS,   // the compression flag of every point
+  N_BUFS = MULTI_PRODUCT + 1
 };
 
 constexpr int N_STREAMS = 8;
@@ -756,6 +762,16 @@ __global__ void compress_pack_kernel(const uint8_t* __restrict__ aff, const uint
   reinterpret_cast<uint32_t*>(out + item * xbytes)[wi] = v;
 }
 
+// the compressed points from the affine points and their flags; xb = 48 (G1) or 96 (G2)
+int pack_dev(const void* aff, const void* flag, void* out, size_t n, int xb) {
+  long long threads = (long long)n * (xb / 4);
+  compress_pack_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, STREAM>>>(
+      (const uint8_t*)aff, (const uint8_t*)flag, (uint8_t*)out, (long long)n, xb);
+  CU(cudaGetLastError());
+  g_ctx.launches++;
+  return 0;
+}
+
 int compress_dev(bool g2, const void* aff, void* out, size_t n) {
   if (n == 0) return 0;
   int rc = ensure(CFLAGS, n);
@@ -764,12 +780,71 @@ int compress_dev(bool g2, const void* aff, void* out, size_t n) {
   VmBuf b[2] = {vb(aff, 2 * xb), vb(dbuf(CFLAGS), 1)};
   rc = launch_named(g2 ? "g2_cflag" : "g1_cflag", n, b, 2);
   if (rc) return rc;
-  long long threads = (long long)n * (xb / 4);
-  compress_pack_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, STREAM>>>(
-      (const uint8_t*)aff, (const uint8_t*)dbuf(CFLAGS), (uint8_t*)out, (long long)n, xb);
+  return pack_dev(aff, dbuf(CFLAGS), out, n, xb);
+}
+
+// ---- signing and public keys (PrivateKey.sign_prehashed / get_public_key, keys.py:119-132) ------------------------
+// sk (n x 32 bytes big-endian, any value) -> the digit records of the g2_sign / g1_pubkey ladders, one thread each
+__global__ void scalar_split_kernel(const uint8_t* __restrict__ sk, uint8_t* __restrict__ out, long long n) {
+  long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n) return;
+  scalar_split(sk + t * 32, out + t * 32);
+}
+
+int split_dev(const void* sk, void* digits, size_t n) {
+  scalar_split_kernel<<<(unsigned)((n + 255) / 256), 256, 0, STREAM>>>((const uint8_t*)sk, (uint8_t*)digits,
+                                                                        (long long)n);
   CU(cudaGetLastError());
   g_ctx.launches++;
   return 0;
+}
+
+// zeroes a device copy of secret data once the work enqueued before it has read it; keeps the first error
+int wipe(int rc, void* p, size_t bytes) {
+  if (!bytes) return rc;
+  cudaError_t e = cudaMemsetAsync(p, 0, bytes, STREAM);
+  if (!rc && e != cudaSuccess) return fail(B200BLS_E_CUDA, "wiping secret data failed: %s", cudaGetErrorString(e));
+  return rc;
+}
+
+// split, then `program` on {extra..., digits, affine out, flags}, then (wire) the compression pack; the digits are
+// zeroed after the program whatever happens
+int digits_pipeline(const char* program, bool g2, bool wire, const void* sk, const VmBuf* extra, int n_extra, void* out,
+                    size_t n) {
+  const size_t w = g2 ? 192 : 96;
+  int rc = ensure(SIGN_DIGITS, 32 * n);
+  if (!rc) rc = ensure(SIGN_FLAGS, n);
+  if (!rc && wire) rc = ensure(SIGN_AFFINE, w * n);
+  if (rc) return rc;
+  void* aff = wire ? dbuf(SIGN_AFFINE) : out;
+  rc = split_dev(sk, dbuf(SIGN_DIGITS), n);
+  if (!rc) {
+    VmBuf b[VM_MAX_BUFS];
+    for (int i = 0; i < n_extra; i++) b[i] = extra[i];
+    b[n_extra] = vb(dbuf(SIGN_DIGITS), 32);
+    b[n_extra + 1] = vb(aff, (long long)w);
+    b[n_extra + 2] = vb(dbuf(SIGN_FLAGS), 1);
+    rc = launch_named(program, n, b, n_extra + 3);
+  }
+  rc = wipe(rc, dbuf(SIGN_DIGITS), 32 * n);
+  if (rc || !wire) return rc;
+  return pack_dev(aff, dbuf(SIGN_FLAGS), out, n, (int)w / 2);
+}
+
+// sk_i * H(mh_i): the SHA stage, the split, g2_sign (hash, psi-split ladder, to_affine, flag), the pack
+int sign_dev(bool wire, const void* sk, const void* mh, void* sig, size_t n) {
+  if (n == 0) return 0;
+  int rc = ensure(SHA_OUT, (size_t)256 * n);
+  if (!rc) rc = sha_stage_dev(mh, dbuf(SHA_OUT), n);
+  if (rc) return rc;
+  VmBuf sha = vb(dbuf(SHA_OUT), 256);
+  return digits_pipeline("g2_sign", true, wire, sk, &sha, 1, sig, n);
+}
+
+// sk_i * G1: the split, g1_pubkey (fixed-base ladder, to_affine, flag), the pack
+int public_key_dev(bool wire, const void* sk, void* pk, size_t n) {
+  if (n == 0) return 0;
+  return digits_pipeline("g1_pubkey", false, wire, sk, nullptr, 0, pk, n);
 }
 
 const char* kFieldOps[] = {"add", "sub", "mul", "sqr", "neg", "inv"};
@@ -1214,6 +1289,32 @@ int b200bls_key_validate_batch(const uint8_t* pts, uint8_t* ok, size_t n) {
 }
 int b200bls_key_validate_batch_dev(const void* pts, void* ok, size_t n) {
   return locked([&] { return point_flags_dev("g1_keyvalidate", false, pts, ok, n); });
+}
+
+// ---- signing and public keys ----------------------------------------------------------------------
+int b200bls_sign_batch(int wire, const uint8_t* sk32, const uint8_t* mh32, uint8_t* sig, size_t n) {
+  if (wire != 0 && wire != 1) return fail(B200BLS_E_ARG, "sign: wire must be 0 (affine) or 1 (compressed)");
+  if (n && (!sk32 || !mh32 || !sig)) return fail(B200BLS_E_ARG, "null buffer");
+  if (n == 0) return 0;
+  HostIO io[3] = {{sk32, nullptr, 32 * n}, {mh32, nullptr, 32 * n}, {nullptr, sig, (wire ? 96 : 192) * n}};
+  return with_staging(io, 3, [&](void** d) { return wipe(sign_dev(wire != 0, d[0], d[1], d[2], n), d[0], 32 * n); });
+}
+int b200bls_sign_batch_dev(int wire, const void* sk32, const void* mh32, void* sig, size_t n) {
+  if (wire != 0 && wire != 1) return fail(B200BLS_E_ARG, "sign: wire must be 0 (affine) or 1 (compressed)");
+  if (n && (!sk32 || !mh32 || !sig)) return fail(B200BLS_E_ARG, "null buffer");
+  return locked([&] { return sign_dev(wire != 0, sk32, mh32, sig, n); });
+}
+int b200bls_public_key_batch(int wire, const uint8_t* sk32, uint8_t* pk, size_t n) {
+  if (wire != 0 && wire != 1) return fail(B200BLS_E_ARG, "public_key: wire must be 0 (affine) or 1 (compressed)");
+  if (n && (!sk32 || !pk)) return fail(B200BLS_E_ARG, "null buffer");
+  if (n == 0) return 0;
+  HostIO io[2] = {{sk32, nullptr, 32 * n}, {nullptr, pk, (wire ? 48 : 96) * n}};
+  return with_staging(io, 2, [&](void** d) { return wipe(public_key_dev(wire != 0, d[0], d[1], n), d[0], 32 * n); });
+}
+int b200bls_public_key_batch_dev(int wire, const void* sk32, void* pk, size_t n) {
+  if (wire != 0 && wire != 1) return fail(B200BLS_E_ARG, "public_key: wire must be 0 (affine) or 1 (compressed)");
+  if (n && (!sk32 || !pk)) return fail(B200BLS_E_ARG, "null buffer");
+  return locked([&] { return public_key_dev(wire != 0, sk32, pk, n); });
 }
 
 // ---- hashing, multi-pairing, verification ----------------------------------------------------
