@@ -150,6 +150,19 @@ int b200bls_miller_product_dev(const void* P, const void* Q, void* out, size_t n
  * prod_i miller(P_i, Q_i), one final exponentiation.  out: 576 bytes. */
 int b200bls_pairing_multi(const uint8_t* P, const uint8_t* Q, uint8_t* out, size_t n);
 int b200bls_pairing_multi_dev(const void* P, const void* Q, void* out, size_t n);
+/* Many fq_ate_pairing_multi products in one device pass: n_groups products
+ * prod_{j in [off[g], off[g+1])} e(P_j, Q_j), one final exponentiation each.
+ * P: total x 96, Q: total x 192 (total = off[n_groups]); off: n_groups + 1 uint64, off[0] = 0, non-decreasing,
+ * total <= 2^32 - 1, n_groups <= 2^31 - 1.
+ * check = 0: out = n_groups x 576 canonical Fq12 bytes (an empty group gives one, as fields_t.py:1117);
+ * check = 1: out = n_groups bytes, 1 iff the product is one (the cheaper final_exp_check).
+ * Other offsets or check values return B200BLS_E_ARG; n_groups = 0 does nothing.  The host form checks the offsets
+ * on the host.  The _dev form takes `off` in device memory as well: its offsets are checked on the device before any
+ * pairing runs, and it synchronises the stream once to read that check and the chunk counts. */
+int b200bls_pairing_multi_batch(int check, const uint8_t* P, const uint8_t* Q, const uint64_t* off,
+                                size_t n_groups, uint8_t* out);
+int b200bls_pairing_multi_batch_dev(int check, const void* P, const void* Q, const void* off,
+                                    size_t n_groups, void* out);
 
 /* ---- curve arithmetic (affine in, affine out; infinity = zero bytes) --------------------------
  * G1 points 96 bytes, G2 points 192 bytes, scalars 32 bytes big-endian (any value < 2^256;

@@ -64,6 +64,8 @@ def _load():
         "b200bls_miller_product_dev": (i32, [vp, vp, vp, sz]),
         "b200bls_pairing_multi": (i32, [vp, vp, vp, sz]),
         "b200bls_pairing_multi_dev": (i32, [vp, vp, vp, sz]),
+        "b200bls_pairing_multi_batch": (i32, [i32, vp, vp, vp, sz, vp]),
+        "b200bls_pairing_multi_batch_dev": (i32, [i32, vp, vp, vp, sz, vp]),
         "b200bls_g1_scalar_mul_batch": (i32, [vp, vp, vp, sz]),
         "b200bls_g1_scalar_mul_batch_dev": (i32, [vp, vp, vp, sz]),
         "b200bls_g2_scalar_mul_batch": (i32, [vp, vp, vp, sz]),

@@ -175,6 +175,31 @@ def pairing_multi(P, Q):
     return out
 
 
+def pairing_multi_batch(P, Q, counts_or_offsets, check=False, offsets=False):
+    """many ate_pairing_multi products in one device pass: group g is the next counts[g] pairs of (P, Q), or with
+    offsets=True the pairs [offsets[g], offsets[g + 1]) -> n x 576 bytes (an empty group gives one), or with check=True
+    n flag bytes, 1 iff the group's product is one"""
+    _lib.init()
+    P, Q, total = _pq(P, Q)
+    v = np.asarray(counts_or_offsets, dtype=np.int64).reshape(-1)
+    if offsets:
+        if v.size == 0:
+            raise ValueError("offsets hold n + 1 entries")
+        off = v
+    else:
+        if (v < 0).any():
+            raise ValueError("negative group size")
+        off = np.concatenate([[0], np.cumsum(v)])
+    if off[-1] != total:
+        raise ValueError("the groups hold %d pairs, P and Q %d" % (off[-1], total))
+    off = np.ascontiguousarray(off.astype(np.uint64))
+    n = off.size - 1
+    out = np.empty(n * (1 if check else 576), dtype=np.uint8)
+    _lib.check(lib.b200bls_pairing_multi_batch(int(bool(check)), ptr(P) if total else None,
+                                               ptr(Q) if total else None, ptr(off), n, ptr(out)))
+    return out
+
+
 def _g(g2):
     return ("g2", 192) if g2 else ("g1", 96)
 

@@ -25,6 +25,16 @@ def ate_pairing_multi(Ps, Qs, ec=None):
     return Fq12(engine.pairing_multi(P, Q).tobytes())
 
 
+def ate_pairing_multi_batch(groups):
+    """[ate_pairing_multi(Ps, Qs) for (Ps, Qs) in groups] in one device pass -> list of Fq12"""
+    groups = [(list(Ps), list(Qs)) for Ps, Qs in groups]
+    packed = [_pack(Ps, Qs) for Ps, Qs in groups]
+    P = b"".join(p for p, _ in packed)
+    Q = b"".join(q for _, q in packed)
+    out = engine.pairing_multi_batch(P, Q, [len(Ps) for Ps, _ in groups]).tobytes()
+    return [Fq12(out[576 * i:576 * (i + 1)]) for i in range(len(groups))]
+
+
 def ate_pairing_batch(Ps, Qs):
     """independent pairings, one per (P_i, Q_i) -> list of Fq12"""
     P, Q = _pack(list(Ps), list(Qs))

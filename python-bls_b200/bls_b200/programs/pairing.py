@@ -418,9 +418,10 @@ def _f12_tree_product(prog, f, nt=128):
     return f
 
 
-def _f12_strided_product(prog):
-    """prologue + body shared by the two product passes: every thread multiplies its strided
-    share of raw SoA Fq12 items (buffer 0) into a persistent accumulator"""
+def _f12_fold(prog):
+    """prologue + body: every thread multiplies the raw SoA Fq12 items (buffer 0) its body
+    iterations visit into a persistent accumulator that starts at one; returns the accumulator
+    at the start of the epilogue"""
     one12 = f12_one(prog)
     acc = [prog.var2(c) for c in one12.coeffs()]
     prog.begin_body()
@@ -431,7 +432,13 @@ def _f12_strided_product(prog):
     for a, v in zip(acc, r.coeffs()):
         prog.assign(a, v)
     prog.begin_epilogue()
-    return _f12_tree_product(prog, F12.from_coeffs(list(acc)))
+    return F12.from_coeffs(list(acc))
+
+
+def _f12_strided_product(prog):
+    """prologue + body shared by the two product passes: every thread multiplies its strided
+    share of raw SoA Fq12 items (buffer 0), then a tree over the CTA"""
+    return _f12_tree_product(prog, _f12_fold(prog))
 
 
 def build_f12_product_pass1():
@@ -452,6 +459,25 @@ def build_f12_product_pass2():
     for k, c in enumerate(tot.coeffs()):
         prog.store2_be48(1, 96 * k, c, block_only=True)
     return prog
+
+
+def build_f12_product_seg(be):
+    """one pass of the batched multi-pairing's segmented product (segmented launch mode, chunk
+    tables from csrc/multi_plan.h): thread t multiplies the raw SoA Fq12 items of chunk t
+    (buffer 0, at most kMultiL of them, read through the index list) starting from one, so an
+    empty chunk gives one.  buffer 1 = one product per chunk: raw SoA (f12_prodseg, the input
+    of the next pass) or 576 big-endian bytes (f12_prodseg_be, the last pass: the input of
+    final_exp / final_exp_check)."""
+    def build():
+        prog = Program("f12_prodseg_be" if be else "f12_prodseg")
+        tot = _f12_fold(prog)
+        for k, c in enumerate(tot.coeffs()):
+            if be:
+                prog.store2_be48(1, 96 * k, c)
+            else:
+                prog.store_raw2(1, k, c)
+        return prog
+    return build
 
 
 def build_miller_only():

@@ -36,6 +36,8 @@ PROGRAMS["miller_raw"] = pairing.build_miller_raw
 PROGRAMS["miller_hash_raw"] = pairing.build_miller_hash_raw
 PROGRAMS["f12_prod1"] = pairing.build_f12_product_pass1
 PROGRAMS["f12_prod2"] = pairing.build_f12_product_pass2
+PROGRAMS["f12_prodseg"] = pairing.build_f12_product_seg(False)
+PROGRAMS["f12_prodseg_be"] = pairing.build_f12_product_seg(True)
 PROGRAMS["hash_to_g2"] = hashg2.build_hash_to_g2
 # single-function parity programs (golden-vector replay of reference functions the hot programs only use inside
 # larger computations); pow is 384 square-and-multiply steps: assembled for the one-CTA-per-SM shape only

@@ -21,6 +21,7 @@
 #include "comm.cuh"
 #include "sha256.cuh"
 #include "gen/vm_isa.h"
+#include "multi_plan.h"
 #include "scalar_split.h"
 #include "vm_launch.h"
 #include "vm_plan.h"
@@ -104,6 +105,14 @@ enum Buf {
   SIGN_DIGITS = MSM_MONT,   // the base-a digits of sk mod n (scalar_split.h): secret, zeroed after the program
   SIGN_AFFINE = MSM_IDX,    // wire output: the affine points before the compression pack
   SIGN_FLAGS = MSM_SEGMENTS,   // the compression flag of every point
+  // pairing_multi_batch_dev calls none of msm_dev, verify_wire_dev, sign_dev, public_key_dev, miller_product_dev, and
+  // none of them calls it: it takes the MSM buffers (and MILLER_RAW for the Miller values)
+  MULTI_TABLES = MSM_OFFSETS,  //   the header (validity, pairs, chunks per pass) and the prefix tables (multi_plan.h)
+  MULTI_SEG = MSM_SEGMENTS,    //   the segment starts of the pass being run
+  MULTI_IDX = MSM_IDX,         //   the index list of the segmented launches
+  MULTI_PARTS = MSM_SEG_SUMS,  //   raw chunk products of the even passes
+  MULTI_PARTS2 = MSM_SCALED,   //   raw chunk products of the odd passes
+  MULTI_FINAL = MSM_MONT,      //   one product per group, big-endian: the input of the final exponentiation
   N_BUFS = MULTI_PRODUCT + 1
 };
 
@@ -599,6 +608,137 @@ int pairing_multi_dev(const void* P, const void* Q, void* out576, size_t n) {
   if (rc) return rc;
   VmBuf b[2] = {vb(dbuf(MULTI_PRODUCT), 576), vb(out576, 576)};
   return launch_named("final_exp", 1, b, 2);
+}
+
+// ---- batched multi-pairing: ragged groups of pairs, one product and one final exponentiation per group ---------------
+// What the host reads back after the scan: whether the offsets are valid, the number of pairs, the chunks of each pass.
+struct MultiHeader {
+  uint32_t bad;
+  uint32_t chunks[kMultiMaxPasses];
+  uint32_t pad;
+  uint64_t total;
+};
+constexpr size_t kMultiHeaderBytes = 64;
+static_assert(sizeof(MultiHeader) <= kMultiHeaderBytes, "multi-pairing header");
+
+// One block: validates the n + 1 offsets and writes the prefix tables of every pass (multi_plan.h).  Thread t owns a
+// contiguous range of groups: their chunk counts, a scan over the threads' sums per pass, then the table entries.
+__global__ void __launch_bounds__(1024) multi_scan_kernel(const uint64_t* __restrict__ off, unsigned long long n,
+                                                          uint32_t* __restrict__ prefix, MultiHeader* __restrict__ hdr) {
+  __shared__ uint32_t part[kMultiMaxPasses][1024];
+  __shared__ int s_bad;
+  const int t = threadIdx.x;
+  if (t == 0) s_bad = 0;
+  __syncthreads();
+  const unsigned long long per = (n + 1023) / 1024;
+  const unsigned long long g0 = min(n, (unsigned long long)t * per), g1 = min(n, g0 + per);
+  uint32_t sum[kMultiMaxPasses] = {}, cnt[kMultiMaxPasses];
+  bool bad = t == 0 && (off[0] != 0 || off[n] > kMultiMaxPairs);
+  for (unsigned long long g = g0; g < g1; g++) {
+    const uint64_t a = off[g], b = off[g + 1];
+    bad = bad || b < a;
+    multi_group_chunks(b - a, cnt);
+#pragma unroll
+    for (int r = 0; r < kMultiMaxPasses; r++) sum[r] += cnt[r];
+  }
+  if (bad) s_bad = 1;
+#pragma unroll
+  for (int r = 0; r < kMultiMaxPasses; r++) part[r][t] = sum[r];
+  __syncthreads();
+  for (int d = 1; d < 1024; d <<= 1) {
+    uint32_t v[kMultiMaxPasses];
+#pragma unroll
+    for (int r = 0; r < kMultiMaxPasses; r++) v[r] = t >= d ? part[r][t - d] : 0;
+    __syncthreads();
+#pragma unroll
+    for (int r = 0; r < kMultiMaxPasses; r++) part[r][t] += v[r];
+    __syncthreads();
+  }
+  uint32_t run[kMultiMaxPasses];
+#pragma unroll
+  for (int r = 0; r < kMultiMaxPasses; r++) run[r] = part[r][t] - sum[r];
+  for (unsigned long long g = g0; g < g1; g++) {
+    multi_group_chunks(off[g + 1] - off[g], cnt);
+#pragma unroll
+    for (int r = 0; r < kMultiMaxPasses; r++) {
+      prefix[r * (n + 1) + g] = run[r];
+      run[r] += cnt[r];
+    }
+  }
+  if (t == 1023) {
+#pragma unroll
+    for (int r = 0; r < kMultiMaxPasses; r++) {
+      prefix[r * (n + 1) + n] = run[r];
+      hdr->chunks[r] = run[r];
+    }
+    hdr->total = off[n];
+    hdr->bad = (uint32_t)s_bad;
+  }
+}
+
+// the segment starts of pass r, one thread per group, and (n_idx > 0) the index list idx[i] = i for i < n_idx
+__global__ void multi_tables_kernel(int r, const uint64_t* __restrict__ off, unsigned long long n,
+                                    const uint32_t* __restrict__ prefix, uint32_t* __restrict__ seg_start,
+                                    uint32_t* __restrict__ idx, unsigned long long n_idx) {
+  const unsigned long long t = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t < n) multi_segments_group(r, t, n, off, prefix, seg_start);
+  if (t < n_idx) idx[t] = (uint32_t)t;
+}
+
+// n_groups products prod_{j in [off[g], off[g + 1])} e(P_j, Q_j) -> out: 576 bytes each (check = false) or one byte,
+// 1 iff the product is one (check = true).  Offsets that are not valid (multi_offsets_bad) are refused before any
+// program runs; the one host synchronisation reads the scan's header.
+int pairing_multi_batch_dev(bool check, const void* P, const void* Q, const uint64_t* off, size_t n_groups, void* out) {
+  if (n_groups == 0) return 0;
+  if (n_groups > kMultiMaxGroups) return fail(B200BLS_E_ARG, "pairing_multi_batch: more than 2^31 - 1 groups");
+  const size_t n = n_groups, rows = (size_t)kMultiMaxPasses * (n + 1);
+  int rc = ensure(MULTI_TABLES, kMultiHeaderBytes + sizeof(uint32_t) * rows);
+  if (rc) return rc;
+  MultiHeader* dhdr = (MultiHeader*)dbuf(MULTI_TABLES);
+  uint32_t* prefix = (uint32_t*)((uint8_t*)dhdr + kMultiHeaderBytes);
+  multi_scan_kernel<<<1, 1024, 0, STREAM>>>(off, n, prefix, dhdr);
+  CU(cudaGetLastError());
+  g_ctx.launches++;
+  MultiHeader h;
+  CU(cudaMemcpyAsync(&h, dhdr, sizeof(h), cudaMemcpyDeviceToHost, STREAM));
+  CU(cudaStreamSynchronize(STREAM));
+  if (h.bad)
+    return fail(B200BLS_E_ARG, "pairing_multi_batch: offsets must start at 0, never decrease and hold at most 2^32 - 1 "
+                               "pairs");
+  const size_t total = (size_t)h.total, c0 = h.chunks[0];
+  const int passes = multi_passes(h.chunks, n);
+  const size_t n_idx = total > c0 ? total : c0;
+  rc = ensure(MILLER_RAW, (size_t)576 * (total ? total : 1));
+  if (!rc) rc = ensure(MULTI_SEG, sizeof(uint32_t) * (c0 + 1));
+  if (!rc) rc = ensure(MULTI_IDX, sizeof(uint32_t) * n_idx);
+  if (!rc && passes > 1) rc = ensure(MULTI_PARTS, (size_t)576 * c0);
+  if (!rc && passes > 2) rc = ensure(MULTI_PARTS2, (size_t)576 * h.chunks[1]);
+  if (!rc) rc = ensure(MULTI_FINAL, (size_t)576 * n);
+  if (rc) return rc;
+  if (total) {
+    VmBuf bm[3] = {vb(P, 96), vb(Q, 192), vb(dbuf(MILLER_RAW), (long long)total)};
+    if ((rc = launch_named("miller_raw", total, bm, 3))) return rc;
+  }
+  uint32_t* seg_start = (uint32_t*)dbuf(MULTI_SEG);
+  uint32_t* idx = (uint32_t*)dbuf(MULTI_IDX);
+  VmBuf in = vb(dbuf(MILLER_RAW), (long long)total);
+  for (int r = 0; r < passes; r++) {
+    const size_t chunks = h.chunks[r], threads = r == 0 && n_idx > n ? n_idx : n;
+    multi_tables_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, STREAM>>>(r, off, n, prefix, seg_start, idx,
+                                                                               r == 0 ? n_idx : 0);
+    CU(cudaGetLastError());
+    g_ctx.launches++;
+    const bool last = r + 1 == passes;
+    const DevProgram* pr = find_program(last ? "f12_prodseg_be" : "f12_prodseg", chunks);
+    if (!pr) return B200BLS_E_PROGRAM;
+    const VmBuf res = last ? vb(dbuf(MULTI_FINAL), 576) : vb(dbuf(r % 2 ? MULTI_PARTS2 : MULTI_PARTS), (long long)chunks);
+    VmBuf bp[2] = {in, res};
+    SegArgs seg = {seg_start, idx};
+    if ((rc = launch_program(*pr, chunks, bp, 2, 0, &seg))) return rc;
+    in = res;
+  }
+  VmBuf bf[2] = {vb(dbuf(MULTI_FINAL), 576), vb(out, check ? 1 : 576)};
+  return launch_named(check ? "final_exp_check" : "final_exp", n, bf, 2);
 }
 
 int sha_stage_dev(const void* hashes, void* out256, size_t n);
@@ -1367,6 +1507,29 @@ int b200bls_pairing_multi(const uint8_t* P, const uint8_t* Q, uint8_t* out, size
 }
 int b200bls_pairing_multi_dev(const void* P, const void* Q, void* out, size_t n) {
   return locked([&] { return pairing_multi_dev(P, Q, out, n); });
+}
+int b200bls_pairing_multi_batch(int check, const uint8_t* P, const uint8_t* Q, const uint64_t* off, size_t n_groups,
+                                uint8_t* out) {
+  if (check != 0 && check != 1) return fail(B200BLS_E_ARG, "pairing_multi_batch: check must be 0 (Fq12) or 1 (is one)");
+  if (n_groups == 0) return 0;
+  if (!off || !out) return fail(B200BLS_E_ARG, "null buffer");
+  if (multi_offsets_bad(off, n_groups))
+    return fail(B200BLS_E_ARG, "pairing_multi_batch: offsets must start at 0, never decrease and hold at most 2^32 - 1 "
+                               "pairs in at most 2^31 - 1 groups");
+  const size_t total = (size_t)off[n_groups];
+  if (total && (!P || !Q)) return fail(B200BLS_E_ARG, "null buffer");
+  HostIO io[4] = {{P, nullptr, 96 * total}, {Q, nullptr, 192 * total}, {off, nullptr, 8 * (n_groups + 1)},
+                  {nullptr, out, (check ? 1 : 576) * n_groups}};
+  return with_staging(io, 4, [&](void** d) {
+    return pairing_multi_batch_dev(check != 0, d[0], d[1], (const uint64_t*)d[2], n_groups, d[3]);
+  });
+}
+int b200bls_pairing_multi_batch_dev(int check, const void* P, const void* Q, const void* off, size_t n_groups,
+                                    void* out) {
+  if (check != 0 && check != 1) return fail(B200BLS_E_ARG, "pairing_multi_batch: check must be 0 (Fq12) or 1 (is one)");
+  if (n_groups == 0) return 0;
+  if (!off || !out) return fail(B200BLS_E_ARG, "null buffer");
+  return locked([&] { return pairing_multi_batch_dev(check != 0, P, Q, (const uint64_t*)off, n_groups, out); });
 }
 int b200bls_verify_batch(const uint8_t* pk, const uint8_t* mh, const uint8_t* sig, uint8_t* ok, size_t n) {
   if (!pk || !mh || !sig || !ok) return fail(B200BLS_E_ARG, "null buffer");
